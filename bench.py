@@ -13,6 +13,10 @@ keeps the rows, and so the total work, fixed instead).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N ...            # the reference itself (numba) on the host cores
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's results, sampled, as .npy
+
+Same arguments, same inputs: the network, the parameters and the lateral inflows are generated from fixed seeds, so
+the files --dump-outputs writes let two builds be compared output for output.
 
 One JSON line on rank 0:
   value      device-resident launches, CUDA events (max over ranks)
@@ -74,7 +78,15 @@ def parse():
     ap.add_argument('--staging', default='auto', choices=['auto', 'registers', 'registers-tiled', 'tma', 'out-reach-major', 'lateral-grouped', 'direct', 'direct-nohw'])
     ap.add_argument('--order', default='growth', choices=['growth', 'level'],
                     help='reach order of the synthetic params file: generator order or sorted by topological level')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed to DIR/discharge.npy and '
+                         'DIR/channel_state.npy (float64, a fixed sample of the reaches, at most 64 MB in all)')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the results of the CUDA arm (--impl b200)')
+    return args
 
 
 def coefficients(k, x, dt_routing, dt_runoff):
@@ -461,6 +473,8 @@ def main():
         dist.all_reduce(t_max, op=dist.ReduceOp.MAX)
     total_ms_max = float(t_max.item())
     value = args.reaches * rows * args.steps / (total_ms_max * 1e-3)
+    if args.dump_outputs:                           # before the checks below reuse d_out
+        dump_outputs(args.dump_outputs, torch, dist, rank, world, down, idx, d_out, d_q, rows, dev)
 
     # ---- summary outputs gathered over NVLink (outside the time loop): outlet discharge of the last step ----
     outlets = torch.from_numpy(np.flatnonzero(local_down < 0)).to(dev)
@@ -554,6 +568,53 @@ def main():
         dist.destroy_process_group()
     if not ok:
         raise SystemExit('bench.py: parity check failed (see "checks" / "e2e.host_equals_device_path")')
+
+
+DUMP_BYTES = 60 << 20    # --dump-outputs: payload of all files together, below 64 MB with the .npy headers
+
+
+def dump_sample(down, rows):
+    """Reaches (indices in params-file order) whose results --dump-outputs writes: every basin outlet, whose discharge
+    carries the whole basin upstream of it, and a seeded uniform sample of the other reaches, as many as keep `rows`
+    discharge values and one state value per reach within DUMP_BYTES.  Depends on the network and `rows` only."""
+    k = DUMP_BYTES // ((rows + 1) * 8)
+    if k < 1:
+        raise SystemExit(f'--dump-outputs: {rows} rows of one reach exceed {DUMP_BYTES} bytes')
+    rng = np.random.default_rng(20261020)
+    outlets = np.flatnonzero(down < 0)
+    if outlets.shape[0] >= k:
+        return np.sort(rng.choice(outlets, k, replace=False))
+    inner = np.flatnonzero(down >= 0)
+    extra = rng.choice(inner, min(k - outlets.shape[0], inner.shape[0]), replace=False)
+    return np.sort(np.concatenate([outlets, extra]))
+
+
+def dump_outputs(out_dir, torch, dist, rank, world, down, idx, d_out, d_q, rows, dev):
+    """What the timed path handed back after its last step -- the discharge of that step's rows and the channel state
+    it left -- at the dump_sample reaches, gathered to rank 0 and written there as DIR/discharge.npy (rows x reaches)
+    and DIR/channel_state.npy (reaches), float64, columns in params-file order."""
+    sample = dump_sample(down, rows)
+    pos = np.flatnonzero(np.isin(idx, sample))                     # this rank's columns of sampled reaches
+    pos_t = torch.from_numpy(pos).to(dev)
+    cols_t = torch.from_numpy(np.searchsorted(sample, idx[pos])).to(dev)
+    buf = torch.zeros((rows + 1, sample.shape[0]), dtype=torch.float64, device=dev)
+    buf[:rows, cols_t] = d_out[:rows, pos_t]
+    buf[rows, cols_t] = d_q[pos_t]
+    if dist is not None:                                           # every sampled reach lives on exactly one rank
+        own = torch.zeros(sample.shape[0], dtype=torch.uint8, device=dev)
+        own[cols_t] = 1
+        parts = [torch.empty_like(buf) for _ in range(world)] if rank == 0 else None
+        owners = [torch.empty_like(own) for _ in range(world)] if rank == 0 else None
+        dist.gather(buf, parts, dst=0)
+        dist.gather(own, owners, dst=0)
+        if rank == 0:
+            for p, o in zip(parts, owners):
+                buf[:, o.bool()] = p[:, o.bool()]
+    if rank == 0:
+        res = buf.cpu().numpy()
+        os.makedirs(out_dir, exist_ok=True)
+        np.save(os.path.join(out_dir, 'discharge.npy'), res[:rows])
+        np.save(os.path.join(out_dir, 'channel_state.npy'), res[rows])
 
 
 def parity_error(got, ref):
