@@ -193,6 +193,40 @@ int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init, int64_t l
                            int lateral_f32, int64_t ldl, void *const *out, int64_t ldo, int out_f32, double *q_final,
                            int64_t ldq, double *q_mean, int64_t T, int64_t substeps, int64_t resample);
 
+/* ---- ensemble statistics ---------------------------------------------------------------------
+ * Per-time-step statistics across ensemble members, computed on the device so that only the statistics cross PCIe
+ * (S rows instead of M member rows per time step).  Every statistic is bit-identical to numpy on the stacked
+ * (members, rows, n) fp64 array:
+ *   RR_STAT_MEAN        np.mean(axis=0): members added in member order, then divided by M
+ *   RR_STAT_STD         np.std(axis=0) (ddof = 0): d = x - mean, d*d added in member order, / M, sqrt
+ *   RR_STAT_MIN / MAX   np.min / np.max
+ *   RR_STAT_PERCENTILE  np.percentile(axis=0, q) with numpy's default 'linear' method, q an integer in [0, 100]
+ * Input contract: no NaN (routed discharge is clamped to >= +0 and never NaN; resample means keep that). */
+#define RR_MAX_STATS 16
+enum { RR_STAT_MEAN = 0, RR_STAT_STD = 1, RR_STAT_MIN = 2, RR_STAT_MAX = 3, RR_STAT_PERCENTILE = 4 };
+typedef struct rr_stats_spec {
+    int32_t n_stats;             /* 1 .. RR_MAX_STATS                                    */
+    int32_t kind[RR_MAX_STATS];  /* RR_STAT_*                                            */
+    int32_t q[RR_MAX_STATS];     /* percentile in [0, 100] of RR_STAT_PERCENTILE entries */
+} rr_stats_spec;
+
+/* The statistics kernel alone, on device pointers: member m, row t, reach i is x[m * member_stride + t * ld + i]
+ * (1 <= n_members <= 64).  out[s] (device pointers, one per statistic) is [rows][ldo], float32 (out_f32 != 0) or
+ * float64; column c shows reach subset[c] (device int32 array; NULL: reach c).  Asynchronous on `stream`. */
+int rr_ensemble_stats_dev(const rr_stats_spec *stats, int32_t n_members, const double *x, int64_t member_stride,
+                          int64_t ld, int64_t rows, int64_t n_out, const int32_t *subset, void *const *out, int64_t ldo,
+                          int out_f32, void *stream);
+
+/* rr_route_ensemble_host with the member outputs reduced on the device: per time chunk, all members are routed into an
+ * fp64 device scratch, averaged over `resample` rows, reduced to the statistics of `stats`, and only those are copied
+ * back: out[s] is a host array [T / resample][ldo] (float32 or float64).  Honours the plan's output subset
+ * (rr_plan_set_output_subset).  Inputs, q_init / ld_init, q_final and q_mean as rr_route_ensemble_host.  The chunk
+ * length follows the free device memory; a call fails when not even one output row of all members fits. */
+int rr_route_ensemble_stats_host(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
+                                 const void *const *lateral, int lateral_f32, int64_t ldl, const rr_stats_spec *stats,
+                                 void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq, double *q_mean,
+                                 int64_t T, int64_t substeps, int64_t resample);
+
 /* Kernel launches issued by this library on this thread since the last reset (bench.py's
  * gpu_launches claim). */
 int64_t rr_launch_count(int reset);

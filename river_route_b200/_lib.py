@@ -36,6 +36,13 @@ class PlanInfo(C.Structure):
                 ('all_fast', C.c_int32), ('narrow_blocks', C.c_int32), ('n_headwaters', C.c_int64), ('n_work', C.c_int64)]
 
 
+MAX_STATS = 16   # RR_MAX_STATS
+
+
+class StatsSpec(C.Structure):
+    _fields_ = [('n_stats', C.c_int32), ('kind', C.c_int32 * MAX_STATS), ('q', C.c_int32 * MAX_STATS)]
+
+
 def _load() -> C.CDLL:
     if not os.path.exists(LIB_PATH):
         raise ImportError(
@@ -70,6 +77,11 @@ def _load() -> C.CDLL:
         'rr_plan_tile_rows': (i64, [vp, i64, i64]),
         'rr_route_ensemble_host': (C.c_int, [vp, C.c_int, f64p, i64, i32, C.POINTER(vp), C.c_int, i64, C.POINTER(vp), i64, C.c_int, f64p, i64,
                                              f64p, i64, i64, i64]),
+        'rr_ensemble_stats_dev': (C.c_int, [C.POINTER(StatsSpec), i32, vp, i64, i64, i64, i64, vp, C.POINTER(vp), i64,
+                                            C.c_int, vp]),
+        'rr_route_ensemble_stats_host': (C.c_int, [vp, C.c_int, f64p, i64, i32, C.POINTER(vp), C.c_int, i64,
+                                                   C.POINTER(StatsSpec), C.POINTER(vp), i64, C.c_int, f64p, i64, f64p, i64,
+                                                   i64, i64]),
         'rr_launch_count': (i64, [C.c_int]),
         'rr_timing_enable': (C.c_int, [C.c_int]),
         'rr_timing_read': (C.c_int, [f64p, c_i64p, C.c_int]),
@@ -99,7 +111,8 @@ EXPORTED_SYMBOLS = (
     'rr_last_error', 'rr_version', 'rr_cuda_available', 'rr_downstream_index', 'rr_label_basins',
     'rr_plan_create', 'rr_plan_destroy', 'rr_plan_get_info', 'rr_plan_set_coefficients', 'rr_route_dev',
     'rr_route_host', 'rr_plan_set_output_subset', 'rr_route_host_ex', 'rr_route_host_typed', 'rr_transform_create', 'rr_transform_set_uh', 'rr_transform_get_uh_state',
-    'rr_transform_destroy', 'rr_runoff_route_host', 'rr_route_ensemble_dev', 'rr_route_ensemble_host', 'rr_plan_tile_rows', 'rr_launch_count', 'rr_timing_enable', 'rr_timing_read', 'rr_uh_convolve_dev', 'rr_uh_convolve_host',
+    'rr_transform_destroy', 'rr_runoff_route_host', 'rr_route_ensemble_dev', 'rr_route_ensemble_host', 'rr_plan_tile_rows',
+    'rr_ensemble_stats_dev', 'rr_route_ensemble_stats_host', 'rr_launch_count', 'rr_timing_enable', 'rr_timing_read', 'rr_uh_convolve_dev', 'rr_uh_convolve_host',
     'rr_weights_transform_dev', 'rr_weights_transform_host', 'rr_plan_read_profile', 'rr_host_alloc', 'rr_host_free', 'rr_synth_forest',
     'rr_plan_get_arrays', 'rr_plan_schedule',
 )

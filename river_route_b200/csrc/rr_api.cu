@@ -919,6 +919,21 @@ struct rr_stream_source {
     int64_t ldx = 0;
 };
 
+// Device copy of the plan's output subset, refreshed when rr_plan_set_output_subset changed it.
+static int upload_subset(rr_plan *p) {
+    rr_device_state *d = p->dev;
+    if (d->out_subset_version == p->out_subset_version) return 0;
+    CK(cudaDeviceSynchronize());
+    if (d->out_subset) CK(cudaFree(d->out_subset));
+    d->out_subset = nullptr;
+    if (!p->out_subset.empty()) {
+        CK(cudaMalloc((void **)&d->out_subset, p->out_subset.size() * sizeof(int32_t)));
+        CK(cudaMemcpy(d->out_subset, p->out_subset.data(), p->out_subset.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    }
+    d->out_subset_version = p->out_subset_version;
+    return 0;
+}
+
 // Host arrays: stream time chunks through two device buffers per direction.
 //   s_in : H2D of chunk c+1        (cudaMemcpy2DAsync, pinned source gives full PCIe rate)
 //   s_comp: [weights -> unit hydrograph ->] route chunk c [-> resample / float32]   (state carried on the device)
@@ -986,16 +1001,7 @@ static int stream_route_impl(rr_plan *p, int mode, double *q_state, double *q_fu
         *cap = need;
         return 0;
     };
-    if (d->out_subset_version != p->out_subset_version) {
-        CK(cudaDeviceSynchronize());
-        if (d->out_subset) CK(cudaFree(d->out_subset));
-        d->out_subset = nullptr;
-        if (!p->out_subset.empty()) {
-            CK(cudaMalloc((void **)&d->out_subset, p->out_subset.size() * sizeof(int32_t)));
-            CK(cudaMemcpy(d->out_subset, p->out_subset.data(), p->out_subset.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-        }
-        d->out_subset_version = p->out_subset_version;
-    }
+    if ((rc = upload_subset(p))) return rc;
     for (int k = 0; k < 2; ++k) {
         if ((rc = grow_bytes(&d->s_inb[k], &d->s_inb_cap[k], need_in))) return rc;
         if ((rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], need_out))) return rc;
@@ -1173,6 +1179,8 @@ static int stream_route(rr_plan *p, int mode, double *q_state, double *q_full, c
 // every member from the same initial state (TransformMuskingum.py:121-126); chunks are double-buffered like the
 // single-member stream (H2D of chunk c+1 | device work of chunk c | D2H of chunk c-1).  The member states stay on the
 // device between chunks; at the end they are copied back and averaged in member order (:145-146).
+// With `stats`, the members' fp64 rows stay on the device and only their statistics (rr_stats.cu) are copied back:
+// out[s] / ldo / out_f32 then describe the statistic arrays, over the plan's output subset.
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) member_mean_kernel(const double *__restrict__ states, int64_t ld, int n_members, int64_t n,
                                                            double *__restrict__ mean) {
@@ -1185,25 +1193,64 @@ __global__ void __launch_bounds__(256) member_mean_kernel(const double *__restri
 
 static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int M, const void *const *lateral, int lat_f32,
                               int64_t ldl, void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq,
-                              double *q_mean, int64_t T, int64_t K, int64_t resample) {
+                              double *q_mean, int64_t T, int64_t K, int64_t resample, const rr_stats_plan *stats = nullptr) {
     if (!p || !q_init || !out || M < 1 || M > RR_MAX_MEMBERS) { rr_set_error("bad ensemble arguments (1..64 members)"); return 100; }
     if (mode == RR_MODE_UNIT) { rr_set_error("ensemble calls support Muskingum / RapidMuskingum"); return 100; }
     const bool has_lat = mode != RR_MODE_MUSKINGUM;
     if (has_lat && !lateral) { rr_set_error("null argument"); return 100; }
     if (T <= 0 || K <= 0 || resample < 1 || T % resample) { rr_set_error("T must be positive and a multiple of the resampling factor"); return 100; }
-    if (!p->out_subset.empty()) { rr_set_error("ensemble calls copy back all river segments (clear the output subset)"); return 100; }
+    if (!stats && !p->out_subset.empty()) { rr_set_error("ensemble calls copy back all river segments (clear the output subset)"); return 100; }
+    if (stats && stats->n_members != M) { rr_set_error("internal: statistics prepared for another member count"); return 101; }
     int rc = ensure_device(p);
     if (rc) return rc;
     rr_device_state *d = p->dev;
     const int64_t n = p->n, ldd = ((n + 31) / 32) * 32;
-    if (ldo < n || (has_lat && ldl < n) || (q_final && ldq < n) || (ld_init != 0 && ld_init < n)) { rr_set_error("leading dimension smaller than n"); return 100; }
+    const int64_t n_out = (stats && !p->out_subset.empty()) ? (int64_t)p->out_subset.size() : n;   // columns copied back
+    const int64_t ldd_out = ((n_out + 31) / 32) * 32;
+    const int n_arrays = stats ? stats->n_stats : M;                                                 // host arrays per row
+    if (ldo < n_out || (has_lat && ldl < n) || (q_final && ldq < n) || (ld_init != 0 && ld_init < n)) { rr_set_error("leading dimension smaller than n"); return 100; }
     const bool pipe = pipeline_ok(p, mode, K);
-    const bool fused = pipe && resample == 1;
+    const bool fused = pipe && resample == 1 && !stats;
     const bool cast_first = has_lat && lat_f32 && !(pipe && K == 1);
     const size_t es_in = lat_f32 ? 4 : 8, es_out = out_f32 ? 4 : 8;
-    // chunk rows: all members of a chunk are resident at once -- transfer buffers (x2), working tiles and scratch
-    const double per_row = (double)M * (double)ldd * (2.0 * es_in + 2.0 * es_out + 16.0 + ((!fused) ? 8.0 : 0.0) + (cast_first ? 8.0 : 0.0));
-    int64_t chunk = std::max<int64_t>(1, (int64_t)((double)(24ll << 30) / per_row));
+    int64_t chunk;
+    if (!stats) {
+        // chunk rows: all members of a chunk are resident at once -- transfer buffers (x2), working tiles and scratch
+        const double per_row = (double)M * (double)ldd * (2.0 * es_in + 2.0 * es_out + 16.0 + ((!fused) ? 8.0 : 0.0) + (cast_first ? 8.0 : 0.0));
+        chunk = std::max<int64_t>(1, (int64_t)((double)(24ll << 30) / per_row));
+    } else {
+        // the longest chunk whose buffers fit the free device memory: what the buffers of this path hold already is
+        // theirs, a larger one must fit next to everything else (one row of all members at 7M reaches is ~12 GB)
+        size_t free_b = 0, total_b = 0;
+        CK(cudaMemGetInfo(&free_b, &total_b));
+        const double ldp = (double)(((p->n_work + 31) / 32) * 32), md = (double)M * (double)ldd;
+        const double caps[] = {(double)d->s_inb_cap[0], (double)d->s_inb_cap[1], (double)d->s_outb_cap[0], (double)d->s_outb_cap[1],
+                               (double)d->s_lat_cap, (double)d->s_route_cap, 8.0 * d->p_lat_cap, 8.0 * d->p_out_cap,
+                               8.0 * d->p_q_cap, (double)d->ens_q_cap};
+        auto extra = [&](int64_t c) {
+            const double tiles = (double)M * ldp * 8.0 * (double)((c + RR_FLAG_ROWS - 1) / RR_FLAG_ROWS * RR_FLAG_ROWS);
+            const double outb = (double)stats->n_stats * (double)(c / resample) * (double)ldd_out * (double)es_out;
+            const double need[] = {has_lat ? md * c * es_in : 0.0, has_lat ? md * c * es_in : 0.0, outb, outb,
+                                   cast_first ? md * c * 8.0 : 0.0, md * c * 8.0, has_lat ? tiles : 0.0, tiles,
+                                   4.0 * M * ldp * 8.0, (M + 2.0) * ldd * 8.0};
+            double more = 0.0;
+            for (int b = 0; b < 10; ++b) more += std::max(0.0, need[b] - caps[b]);
+            return more;
+        };
+        const double room = 0.92 * (double)free_b - (double)(256ll << 20);
+        int64_t lo = 0, hi = T;   // largest chunk in [resample, T] with extra(chunk) <= room
+        while (lo < hi) {
+            const int64_t mid = (lo + hi + 1) / 2;
+            if (extra(mid) <= room) lo = mid; else hi = mid - 1;
+        }
+        if (lo < resample) {
+            rr_set_error("ensemble statistics: one output row of all " + std::to_string(M) + " members (" +
+                         std::to_string((long long)(extra(resample) / 1e6)) + " MB of device buffers) does not fit in the " +
+                         std::to_string((long long)(free_b / 1000000)) + " MB of free device memory");
+            return 100;
+        }
+        chunk = lo;
+    }
     if (const char *env = getenv("RR_STREAM_CHUNK_ROWS")) chunk = std::max(1, atoi(env));
     const int64_t unit = pipe ? RR_FLAG_ROWS : 8;
     if (chunk >= unit) chunk = chunk / unit * unit;
@@ -1219,11 +1266,13 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         *cap = need;
         return 0;
     };
-    const size_t in_member = (size_t)chunk * ldd * es_in, out_member = (size_t)rows_out_max * ldd * es_out;
+    // out_member: one host array's rows of a chunk (a member's discharge, or one statistic)
+    const size_t in_member = (size_t)chunk * ldd * es_in, out_member = (size_t)rows_out_max * ldd_out * es_out;
     for (int k = 0; k < 2; ++k) {
         if (has_lat && (rc = grow_bytes(&d->s_inb[k], &d->s_inb_cap[k], in_member * M))) return rc;
-        if ((rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], out_member * M))) return rc;
+        if ((rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], out_member * n_arrays))) return rc;
     }
+    if (stats && (rc = upload_subset(p))) return rc;
     const size_t f64_member = (size_t)chunk * ldd * 8;
     if (cast_first && (rc = grow_bytes((void **)&d->s_lat, &d->s_lat_cap, f64_member * M))) return rc;
     if (!fused && (rc = grow_bytes((void **)&d->s_route, &d->s_route_cap, f64_member * M))) return rc;
@@ -1267,13 +1316,21 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
             lat_m[m] = (const double *)in;
             out_m[m] = fused ? nullptr : d->s_route + (f64_member / 8) * m;
             qs_m[m] = d_qm + (size_t)m * ldd;
-            spec[m].dst = (char *)d->s_outb[k] + out_member * m; spec[m].f32 = out_f32; spec[m].ld = ldd;
+            spec[m].dst = (char *)d->s_outb[k] + out_member * m; spec[m].f32 = out_f32; spec[m].ld = ldd_out;
             spec[m].subset = nullptr; spec[m].n_out = n;
         }
         rc = route_any(p, mode, M, d_q0, has_lat ? lat_m : nullptr, ldd, out_m, ldd, qs_m, nullptr, rows, K, c == 0 && shared_init, c == n_chunks - 1,
                        d->s_comp, fused ? spec : nullptr, (has_lat && lat_f32 && !cast_first) ? 1 : 0);
         if (rc) return rc;
-        if (!fused) {
+        if (stats) {
+            // the members' fp64 rows in s_route -> resample -> statistics, one launch
+            void *dst[RR_MAX_STATS];
+            for (int s = 0; s < stats->n_stats; ++s) dst[s] = (char *)d->s_outb[k] + out_member * s;
+            rr_timer tm(3, d->s_comp);
+            rc = rr_stats_launch(*stats, d->s_route, (int64_t)(f64_member / 8), ldd, (int)resample, rows_out, n_out,
+                                 p->out_subset.empty() ? nullptr : d->out_subset, dst, ldd_out, out_f32, d->s_comp);
+            if (rc) return rc;
+        } else if (!fused) {
             for (int m = 0; m < M; ++m) {
                 dim3 g((unsigned)((n + 255) / 256), (unsigned)rows_out);
                 if (out_f32) finish_output<float><<<g, 256, 0, d->s_comp>>>(out_m[m], ldd, (float *)spec[m].dst, ldd, n, (int)resample, nullptr);
@@ -1284,9 +1341,10 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         }
         CK(cudaEventRecord(d->ev_comp[k], d->s_comp));
         CK(cudaStreamWaitEvent(d->s_out, d->ev_comp[k], 0));
-        for (int m = 0; m < M; ++m)
-            CK(cudaMemcpy2DAsync((char *)out[m] + (size_t)(c * chunk / resample) * ldo * es_out, (size_t)ldo * es_out, spec[m].dst,
-                                 (size_t)ldd * es_out, (size_t)n * es_out, rows_out, cudaMemcpyDeviceToHost, d->s_out));
+        for (int a = 0; a < n_arrays; ++a)
+            CK(cudaMemcpy2DAsync((char *)out[a] + (size_t)(c * chunk / resample) * ldo * es_out, (size_t)ldo * es_out,
+                                 (char *)d->s_outb[k] + out_member * a, (size_t)ldd_out * es_out, (size_t)n_out * es_out, rows_out,
+                                 cudaMemcpyDeviceToHost, d->s_out));
         CK(cudaEventRecord(d->ev_out[k], d->s_out));
         if (c + 1 < n_chunks && (rc = copy_in(c + 1))) return rc;
     }
@@ -1303,12 +1361,8 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
     return 0;
 }
 
-extern "C" int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
-                                      const void *const *lateral, int lateral_f32, int64_t ldl, void *const *out, int64_t ldo,
-                                      int out_f32, double *q_final, int64_t ldq, double *q_mean, int64_t T, int64_t substeps,
-                                      int64_t resample) {
-    const int rc = ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32, q_final, ldq, q_mean,
-                                      T, substeps, resample);
+// failed ensemble calls: earlier chunks' copies may still use the caller's arrays; let them finish, keep the message
+static int ensemble_settle(rr_plan *p, int rc) {
     if (rc && p && p->dev) {
         const std::string msg = rr_last_error();
         cudaDeviceSynchronize();
@@ -1316,6 +1370,27 @@ extern "C" int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init
         rr_set_error(msg);
     }
     return rc;
+}
+
+extern "C" int rr_route_ensemble_stats_host(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
+                                            const void *const *lateral, int lateral_f32, int64_t ldl, const rr_stats_spec *stats,
+                                            void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq,
+                                            double *q_mean, int64_t T, int64_t substeps, int64_t resample) {
+    rr_stats_plan sp;
+    int rc = rr_stats_prepare(stats, n_members, &sp);
+    if (rc) return rc;
+    for (int s = 0; out && s < sp.n_stats; ++s)
+        if (!out[s]) { rr_set_error("null output array"); return 100; }
+    return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
+                                                 q_final, ldq, q_mean, T, substeps, resample, &sp));
+}
+
+extern "C" int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
+                                      const void *const *lateral, int lateral_f32, int64_t ldl, void *const *out, int64_t ldo,
+                                      int out_f32, double *q_final, int64_t ldq, double *q_mean, int64_t T, int64_t substeps,
+                                      int64_t resample) {
+    return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
+                                                 q_final, ldq, q_mean, T, substeps, resample));
 }
 
 extern "C" int rr_plan_set_output_subset(rr_plan *p, int64_t n_sub, const int32_t *idx) {

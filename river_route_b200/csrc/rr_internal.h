@@ -88,3 +88,14 @@ void rr_decode_ticket(const rr_plan &p, const rr_schedule &s, int64_t n_tiles, i
                       int32_t *block, int32_t *tile);
 
 void rr_device_release(rr_plan *p);  // frees p->dev (rr_api.cu)
+
+// rr_stats.cu: a validated rr_stats_spec with the percentile positions resolved for M members
+struct rr_stats_plan {
+    int32_t n_stats = 0, n_members = 0, sort = 0;
+    int32_t kind[RR_MAX_STATS] = {}, lo[RR_MAX_STATS] = {}, hi[RR_MAX_STATS] = {};
+    double g[RR_MAX_STATS] = {};
+};
+int rr_stats_prepare(const rr_stats_spec *spec, int32_t n_members, rr_stats_plan *out);
+// out[s] + t * ldo + c = statistic s of row t: the members' rows t*k .. t*k+k-1 averaged first (k = resample)
+int rr_stats_launch(const rr_stats_plan &sp, const double *x, int64_t member_stride, int64_t ld, int k, int64_t rows_out,
+                    int64_t n_out, const int32_t *subset, void *const *out, int64_t ldo, int out_f32, void *stream);

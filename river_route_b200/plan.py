@@ -15,6 +15,7 @@ from . import _lib
 from ._lib import lib, check
 
 MODE_MUSKINGUM, MODE_RAPID, MODE_UNIT = 0, 1, 2
+_STAT_KINDS = {'mean': 0, 'std': 1, 'min': 2, 'max': 3}   # RR_STAT_*; 'pQ' is RR_STAT_PERCENTILE (4) with q = Q
 
 
 def downstream_index(river_ids, downstream_ids) -> np.ndarray:
@@ -52,6 +53,55 @@ def label_basins(down: np.ndarray, n_parts: int = 0):
     check(lib.rr_label_basins(down.shape[0], _lib.as_i32p(down), _lib.as_i32p(basin), C.byref(nb), int(n_parts),
                               _lib.as_i32p(part) if part is not None else None))
     return basin, int(nb.value), part
+
+
+def parse_statistics(names) -> list:
+    """
+    Ensemble statistic names -> ``[(name, kind, q)]``: ``'mean'``, ``'std'`` (population, ddof=0), ``'min'``, ``'max'``
+    and percentiles ``'p0'`` .. ``'p100'`` (integer q, numpy's default 'linear' method).  At most 16, no duplicates;
+    anything else raises ``ValueError``.
+    """
+    if isinstance(names, str):
+        names = [names]
+    names = list(names)
+    if not 1 <= len(names) <= _lib.MAX_STATS:
+        raise ValueError(f'between 1 and {_lib.MAX_STATS} ensemble statistics, got {len(names)}')
+    out = []
+    for name in names:
+        if not isinstance(name, str):
+            raise ValueError(f'ensemble statistic names are strings, got {name!r}')
+        if name in _STAT_KINDS:
+            out.append((name, _STAT_KINDS[name], 0))
+        elif name[:1] == 'p' and name[1:].isdigit() and str(int(name[1:])) == name[1:] and int(name[1:]) <= 100:
+            out.append((name, 4, int(name[1:])))
+        else:
+            raise ValueError(f"unknown ensemble statistic {name!r}: use 'mean', 'std', 'min', 'max' or 'p0' .. 'p100'")
+    if len({o[0] for o in out}) != len(out):
+        raise ValueError(f'duplicate ensemble statistics in {names}')
+    return out
+
+
+def _stats_spec(names):
+    spec = _lib.StatsSpec()
+    parsed = parse_statistics(names)
+    spec.n_stats = len(parsed)
+    for s, (_, kind, q) in enumerate(parsed):
+        spec.kind[s], spec.q[s] = kind, q
+    return spec
+
+
+def ensemble_stats_dev(stats, n_members: int, x_ptr: int, member_stride: int, ld: int, rows: int, n_out: int,
+                       out_ptrs, ldo: int, out_f32: bool, subset_ptr: int = 0, stream: int = 0) -> None:
+    """The statistics kernel alone on device pointers (``rr_ensemble_stats_dev``): member m, row t, reach i is
+    ``x[m * member_stride + t * ld + i]``; ``out_ptrs[s]`` is (rows, ldo) float32 / float64 of statistic ``stats[s]``;
+    column c shows reach ``subset[c]`` (int32 device array) or reach c.  Asynchronous on ``stream``."""
+    spec = _stats_spec(stats)
+    if len(out_ptrs) != spec.n_stats:
+        raise ValueError('one output array per statistic')
+    arr = C.c_void_p * spec.n_stats
+    check(lib.rr_ensemble_stats_dev(C.byref(spec), int(n_members), C.c_void_p(x_ptr), int(member_stride), int(ld), int(rows),
+                                    int(n_out), C.c_void_p(subset_ptr or None), arr(*out_ptrs), int(ldo), int(bool(out_f32)),
+                                    C.c_void_p(stream or None)))
 
 
 def down_from_csc(indptr, indices, n: int) -> np.ndarray:
@@ -265,6 +315,51 @@ class Plan:
                                          arr(*[o.ctypes.data for o in outs]), _lib.rows_ld(outs[0]), int(odt == np.float32),
                                          _lib.as_f64p(q_final) if q_final is not None else None, self.n,
                                          _lib.as_f64p(q_mean), T, int(substeps), resample))
+        return q_mean
+
+    def route_ensemble_stats_host(self, mode: int, q_init: np.ndarray, laterals, stats, outs, substeps: int,
+                                  resample: int = 1, q_final: np.ndarray | None = None):
+        """
+        As ``route_ensemble_host`` -- same members, inputs, state chaining, ``q_final`` and returned member-mean state --
+        but the members' discharge stays on the device: per time chunk it is averaged over ``resample`` rows and reduced
+        to the statistics named in ``stats`` (see ``parse_statistics``), and only those cross PCIe.  ``outs[s]`` is
+        (T / resample, n_out) float32 or float64 (all the same dtype) for statistic ``stats[s]``; n_out follows the
+        output subset (``set_output_subset``).  Every statistic equals numpy on the stacked fp64 member outputs bit for
+        bit (``np.mean`` / ``np.std`` / ``np.min`` / ``np.max`` / ``np.percentile`` over axis 0).
+        """
+        spec = _stats_spec(stats)
+        M = len(laterals) if laterals is not None else 0
+        if mode == MODE_MUSKINGUM:
+            raise ValueError('ensemble statistics need lateral inflows (RapidMuskingum members)')
+        if not 1 <= M <= 64:
+            raise ValueError('ensemble statistics need 1 to 64 members')
+        if len(outs) != spec.n_stats:
+            raise ValueError('one output array per statistic')
+        if q_init.dtype != np.float64 or not q_init.flags.c_contiguous or q_init.shape not in ((self.n,), (M, self.n)):
+            raise ValueError('q_init must be a contiguous float64 (n,) vector or (members, n) array')
+        ld_init = self.n if q_init.ndim == 2 else 0
+        resample = int(resample)
+        n_out = self.n_out
+        T = outs[0].shape[0] * resample
+        odt = outs[0].dtype
+        for o in outs:
+            if o.dtype != odt or odt not in (np.float64, np.float32) or o.shape != (T // resample, n_out) or \
+                    _lib.rows_ld(o) != _lib.rows_ld(outs[0]):
+                raise ValueError('statistic arrays must share dtype (float64 / float32), shape (T / resample, n_out) and row stride')
+        ldt = laterals[0].dtype
+        for a in laterals:
+            if a.dtype != ldt or ldt not in (np.float64, np.float32) or a.shape != (T, self.n) or \
+                    _lib.rows_ld(a) != _lib.rows_ld(laterals[0]):
+                raise ValueError('lateral arrays must share dtype (float64 / float32), shape (T, n) and row stride')
+        if q_final is not None and (q_final.dtype != np.float64 or q_final.shape != (M, self.n) or not q_final.flags.c_contiguous):
+            raise ValueError('q_final must be a contiguous float64 (members, n) array')
+        q_mean = np.empty(self.n, dtype=np.float64)
+        arr_m, arr_s = C.c_void_p * M, C.c_void_p * spec.n_stats
+        check(lib.rr_route_ensemble_stats_host(
+            self._h, int(mode), _lib.as_f64p(q_init), ld_init, M, arr_m(*[a.ctypes.data for a in laterals]),
+            int(ldt == np.float32), _lib.rows_ld(laterals[0]), C.byref(spec), arr_s(*[o.ctypes.data for o in outs]),
+            _lib.rows_ld(outs[0]), int(odt == np.float32), _lib.as_f64p(q_final) if q_final is not None else None, self.n,
+            _lib.as_f64p(q_mean), T, int(substeps), resample))
         return q_mean
 
     def tile_rows(self, T: int, substeps: int = 1) -> int:

@@ -18,7 +18,7 @@ from typing import Any, Callable, Iterator
 import numpy as np
 import pandas as pd
 
-from .plan import MODE_MUSKINGUM, MODE_RAPID, MODE_UNIT, Plan, downstream_index
+from .plan import MODE_MUSKINGUM, MODE_RAPID, MODE_UNIT, Plan, downstream_index, parse_statistics
 from .runoff import runoff_to_qlateral
 from .uhkernels import UnitHydrograph
 
@@ -383,11 +383,12 @@ class Muskingum:
         with self._open_discharge_file(dates, q_array.shape[1], q_file, routed_file) as out:
             out.write_rows(0, q_array)
 
-    def _open_discharge_file(self, dates, n_cols, q_file, routed_file=''):
+    def _open_discharge_file(self, dates, n_cols, q_file, routed_file='', statistics=None):
         """The same file, opened for writing row slabs as they come back from the GPU (streamed runs)."""
         ids = getattr(self, 'river_ids_all', self.river_ids) if getattr(self, '_output_idx', None) is None \
             else self.river_ids[self._output_idx]
-        return _DischargeFile(q_file, dates, ids, n_cols, self.cfg.var_river_id, self.cfg.var_discharge, routed_file)
+        return _DischargeFile(q_file, dates, ids, n_cols, self.cfg.var_river_id, self.cfg.var_discharge, routed_file,
+                              statistics)
 
 
 class TransformMuskingum(Muskingum):
@@ -395,6 +396,21 @@ class TransformMuskingum(Muskingum):
     _ROUTER_REQUIRED_CONFIGS = ()
     _as_volumes = False
     _mode = MODE_RAPID
+    _ensemble_stats = None
+
+    def set_ensemble_statistics(self, path, statistics=('mean', 'std', 'min', 'max', 'p25', 'p50', 'p75')):
+        """
+        Extension: in ``runoff_processing_mode='ensemble'`` with ``qlateral_files``, write per-time-step statistics
+        across the members to ONE netCDF at ``path`` instead of one discharge file per member.  The statistics are
+        computed on the device, so only they cross PCIe.  The file has the discharge files' time / river-id layout
+        (after the ``dt_discharge`` resample, honouring ``set_output_rivers``) and one float32 variable
+        ``<var_discharge>_<stat>`` per statistic (e.g. ``Q_mean``, ``Q_p25``; percentiles carry a ``percentile``
+        attribute).  ``statistics``: ``'mean'``, ``'std'`` (ddof=0), ``'min'``, ``'max'``, ``'p0'`` .. ``'p100'``; each
+        equals numpy's over the members' fp64 discharge, cast to float32.  The final channel state is the member mean,
+        as without statistics.  ``path=None`` switches back to member files.
+        """
+        self._ensemble_stats = None if path is None else (str(path), parse_statistics(statistics))
+        return self
 
     def _qlateral_generator(self) -> Iterator[tuple]:
         """Yields (dates, (T, n) fp64 lateral array, input file, output file) per input file (:30-51)."""
@@ -421,6 +437,23 @@ class TransformMuskingum(Muskingum):
             raise ValueError('Provide qlateral_files or grid_runoff_files with grid_weights_file')
         if len(self.cfg.discharge_files) != len(qlateral) + len(self.cfg.grid_runoff_files or []):
             raise ValueError('Number of resolved discharge output files must match number of input files')
+        if self._ensemble_stats is not None:
+            self._validate_ensemble_statistics()
+
+    def _validate_ensemble_statistics(self):
+        cfg = self.cfg
+        if cfg.runoff_processing_mode != 'ensemble':
+            raise ValueError("set_ensemble_statistics needs runoff_processing_mode='ensemble'")
+        if self._mode == MODE_UNIT:
+            raise ValueError('set_ensemble_statistics is not available for UnitMuskingum')
+        if not cfg.qlateral_files:
+            raise ValueError('set_ensemble_statistics needs qlateral_files (grid_runoff_files ensembles are not supported)')
+        if self._writer is not None:
+            raise ValueError('set_ensemble_statistics writes its own file: it cannot be combined with set_write_discharges')
+        if self._shard is not None and self._shard.world > 1:
+            raise ValueError('set_ensemble_statistics is not available in basin-sharded runs')
+        if len(cfg.qlateral_files) > 64:
+            raise ValueError(f'set_ensemble_statistics supports at most 64 members, got {len(cfg.qlateral_files)}')
 
     def _set_network_and_time_dependent_vectors(self, dates):
         """Time bookkeeping of TransformMuskingum.py:66-106; the device coefficients are refreshed only when the
@@ -466,6 +499,8 @@ class TransformMuskingum(Muskingum):
         ``_qlateral_generator`` gets the reference's sequence on fp64 host arrays instead.
         """
         self._ensemble_member_states = []
+        if self._ensemble_stats is not None:
+            return self._execute_ensemble_statistics()
         device_tail = _is_stock(self, '_router', TransformMuskingum)
         if (device_tail and self.cfg.qlateral_files and _is_stock(self, '_qlateral_generator', TransformMuskingum)
                 and _is_stock(self, '_route_lateral', TransformMuskingum, UnitMuskingum)):
@@ -611,6 +646,79 @@ class TransformMuskingum(Muskingum):
         self._ensemble_member_states = list(states)
         # one group: the device mean (member order, then / M) is the answer; several groups: numpy over all members
         self.channel_state = mean if G == M else np.array(self._ensemble_member_states).mean(axis=0)   # :145-146
+
+    def _execute_ensemble_statistics(self):
+        """
+        ``set_ensemble_statistics``: every qlateral file is one member, all start from the same channel state, and each
+        time slab of ALL members is routed and reduced by one ``Plan.route_ensemble_stats_host`` call (statistics need
+        every member of a time step in the same call, so the work is ordered time slab first).  Slab rows come from
+        RR_ROUTER_SLAB_BYTES over all members; reads and writes run on the thread pool around the device call.
+        """
+        from concurrent.futures import ThreadPoolExecutor
+        path, parsed = self._ensemble_stats
+        cfg = self.cfg
+        M = len(cfg.qlateral_files)
+        names = [p[0] for p in parsed]
+        n, S = self.n, len(parsed)
+        srcs = []
+        try:
+            for lat_file in cfg.qlateral_files:
+                srcs.append(_LateralFile(lat_file))
+            dates = srcs[0].dates
+            self._set_network_and_time_dependent_vectors(dates)
+            T = self.num_runoff_steps
+            k = self.num_runoff_steps_per_discharge if self.dt_discharge > self.dt_runoff else 1
+            for src, lat_file in zip(srcs, cfg.qlateral_files):
+                self.logger.info(f'Routing qlateral: {lat_file}')
+                self._check_lateral_shape(src.shape, n)
+                if src.dates.shape != dates.shape or (len(dates) > 1 and src.dates[1] - src.dates[0] != dates[1] - dates[0]):
+                    raise ValueError('ensemble members must have the same number of time steps and time step')
+            dtype = srcs[0].dtype if all(s_.dtype == srcs[0].dtype for s_ in srcs) else np.dtype(np.float64)
+            if os.environ.get('RR_ROUTER_SLAB_ROWS'):
+                rows = int(os.environ['RR_ROUTER_SLAB_ROWS'])
+            else:
+                rows = int(float(os.environ.get('RR_ROUTER_SLAB_BYTES', 2 << 30)) // max(1, M * n * dtype.itemsize))
+            unit = int(np.lcm(16, k)) if rows >= np.lcm(16, k) else k      # at least one dt_discharge interval
+            slab = min(T, max(unit, rows // unit * unit))
+            starts = list(range(0, T, slab))
+            lat = [[self._pinned(('elat', b, m), (slab, n), dtype) for m in range(M)] for b in range(2)]
+            out = [[self._pinned(('estat', b, s), (slab // k, self._n_out), np.float32) for s in range(S)] for b in range(2)]
+            states = np.empty((M, n), dtype=np.float64)
+            q_members = self.channel_state.astype(np.float64, copy=True)
+            out_file = self._open_discharge_file(dates[::k] if k > 1 else dates, self._n_out, path,
+                                                 ', '.join(str(f) for f in cfg.qlateral_files), statistics=parsed)
+            with out_file, ThreadPoolExecutor(max_workers=4) as pool:
+                def read(s_):
+                    t0, t1 = starts[s_], min(T, starts[s_] + slab)
+                    list(pool.map(lambda m: srcs[m].read(t0, t1, lat[s_ % 2][m]), range(M)))
+                    return t1 - t0
+
+                def write(r0, outs):
+                    for s_, o in enumerate(outs):
+                        out_file.write_rows(r0, o, s_)
+                nxt = pool.submit(read, 0)
+                pending = [None, None]
+                for s_ in range(len(starts)):
+                    rows = nxt.result()
+                    if s_ + 1 < len(starts):
+                        nxt = pool.submit(read, s_ + 1)
+                    if pending[s_ % 2] is not None:
+                        pending[s_ % 2].result()
+                    out_s = [a[:rows // k] for a in out[s_ % 2]]
+                    # later slabs start from the members' own states (q_members is states once the first slab is done)
+                    mean = self.plan.route_ensemble_stats_host(self._mode, q_members, [a[:rows] for a in lat[s_ % 2]], names,
+                                                               out_s, self.num_routing_steps_per_runoff, resample=k,
+                                                               q_final=states)
+                    q_members = states
+                    pending[s_ % 2] = pool.submit(write, starts[s_] // k, out_s)
+                for f in pending:
+                    if f is not None:
+                        f.result()
+        finally:
+            for src in srcs:
+                src.close()
+        self._ensemble_member_states = list(states)
+        self.channel_state = mean                      # member-order mean, then / M (TransformMuskingum.py:145-146)
 
     def _slab_rows(self, T, k, row_bytes):
         """Rows per slab: about RR_ROUTER_SLAB_BYTES (2 GiB) of lateral inflows, whole 16-row groups of the device
@@ -917,7 +1025,9 @@ class UnitMuskingum(TransformMuskingum):
 class _DischargeFile:
     """Discharge netCDF with the reference's layout (Muskingum.py:337-351), written in row slabs."""
 
-    def __init__(self, path, dates, river_ids, n_cols, var_river_id, var_discharge, routed_file=''):
+    def __init__(self, path, dates, river_ids, n_cols, var_river_id, var_discharge, routed_file='', statistics=None):
+        """``statistics`` (``[(name, kind, q)]`` of ``plan.parse_statistics``): one variable ``<var_discharge>_<name>``
+        per ensemble statistic instead of the one discharge variable."""
         from . import ncio
         self.ds = ncio.open_nc(path, 'w')
         ds = self.ds
@@ -929,15 +1039,21 @@ class _DischargeFile:
         tv[:] = (dates - dates[0]).astype('timedelta64[s]').astype(np.int64)
         iv = ds.createVariable(var_river_id, 'i4', (var_river_id,))
         iv[:] = np.asarray(river_ids).astype(np.int32)
-        qv = ds.createVariable(var_discharge, 'f4', ('time', var_river_id))
-        qv.long_name = 'Discharge at catchment outlet'
-        qv.standard_name = 'discharge'
-        qv.aggregation_method = 'mean'
-        qv.units = 'm3 s-1'
-        self.qv = qv
+        self.vars = []
+        for name, kind, q in statistics or [(None, None, None)]:
+            qv = ds.createVariable(var_discharge if name is None else f'{var_discharge}_{name}', 'f4', ('time', var_river_id))
+            qv.long_name = 'Discharge at catchment outlet' if name is None else \
+                f'Ensemble {name} of the discharge at catchment outlet'
+            qv.standard_name = 'discharge'
+            qv.aggregation_method = 'mean'
+            qv.units = 'm3 s-1'
+            if kind == 4:
+                qv.percentile = q
+            self.vars.append(qv)
+        self.qv = self.vars[0]
 
-    def write_rows(self, t0, rows):
-        self.qv[t0:t0 + rows.shape[0], :] = rows
+    def write_rows(self, t0, rows, var=0):
+        self.vars[var][t0:t0 + rows.shape[0], :] = rows
 
     def close(self):
         if self.ds is not None:
