@@ -201,14 +201,22 @@ int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init, int64_t l
  *   RR_STAT_STD         np.std(axis=0) (ddof = 0): d = x - mean, d*d added in member order, / M, sqrt
  *   RR_STAT_MIN / MAX   np.min / np.max
  *   RR_STAT_PERCENTILE  np.percentile(axis=0, q) with numpy's default 'linear' method, q an integer in [0, 100]
- * Input contract: no NaN (routed discharge is clamped to >= +0 and never NaN; resample means keep that). */
+ *   RR_STAT_EXCEED      np.mean(x > thr[q], axis=0): the fraction of members strictly above the reach's threshold in
+ *                       row q of the thresholds (x == thr does not count; a NaN threshold is never exceeded: 0.0)
+ * Input contract: no NaN (routed discharge is clamped to >= +0 and never NaN; resample means keep that).
+ * Horizon peaks (the _ex forms): per statistic and column, the maximum over the output rows and the first row where
+ * it occurs, i.e. rows.max(axis=0) and rows.argmax(axis=0) of the fp64 statistic rows (ties: the earliest row). */
 #define RR_MAX_STATS 16
-enum { RR_STAT_MEAN = 0, RR_STAT_STD = 1, RR_STAT_MIN = 2, RR_STAT_MAX = 3, RR_STAT_PERCENTILE = 4 };
+enum { RR_STAT_MEAN = 0, RR_STAT_STD = 1, RR_STAT_MIN = 2, RR_STAT_MAX = 3, RR_STAT_PERCENTILE = 4, RR_STAT_EXCEED = 5 };
 typedef struct rr_stats_spec {
-    int32_t n_stats;             /* 1 .. RR_MAX_STATS                                    */
-    int32_t kind[RR_MAX_STATS];  /* RR_STAT_*                                            */
-    int32_t q[RR_MAX_STATS];     /* percentile in [0, 100] of RR_STAT_PERCENTILE entries */
+    int32_t n_stats;             /* 1 .. RR_MAX_STATS                                                            */
+    int32_t kind[RR_MAX_STATS];  /* RR_STAT_*                                                                    */
+    int32_t q[RR_MAX_STATS];     /* percentile in [0, 100] of RR_STAT_PERCENTILE entries; threshold row of EXCEED */
 } rr_stats_spec;
+
+/* Per-river thresholds (e.g. return-period flows) for RR_STAT_EXCEED in params-file (user) order: host [n_thr][ldt],
+ * ldt >= n, copied; uploaded to the plan's device lazily and versioned like the output subset.  n_thr = 0 clears. */
+int rr_plan_set_thresholds(rr_plan *p, int32_t n_thr, const double *thr, int64_t ldt);
 
 /* The statistics kernel alone, on device pointers: member m, row t, reach i is x[m * member_stride + t * ld + i]
  * (1 <= n_members <= 64).  out[s] (device pointers, one per statistic) is [rows][ldo], float32 (out_f32 != 0) or
@@ -216,6 +224,17 @@ typedef struct rr_stats_spec {
 int rr_ensemble_stats_dev(const rr_stats_spec *stats, int32_t n_members, const double *x, int64_t member_stride,
                           int64_t ld, int64_t rows, int64_t n_out, const int32_t *subset, void *const *out, int64_t ldo,
                           int out_f32, void *stream);
+
+/* rr_ensemble_stats_dev plus thresholds and running peaks.  thr: device [n_thr][ldt], indexed by reach (column c reads
+ * thr[q * ldt + subset[c]]); needed by RR_STAT_EXCEED entries, NULL otherwise.  peak / peak_row: device [n_stats][ldk]
+ * fp64 / int32, read and updated: where a statistic's value at row t is strictly greater than peak[s][c], peak[s][c]
+ * becomes that value and peak_row[s][c] becomes row0 + t.  Start peak at -inf; launches over consecutive rows with
+ * row0 = the global index of each launch's first row then give the maximum over all of them and its first row.  out
+ * may be NULL (no per-step rows) when peak is given; peak needs peak_row.  No atomics: the result is deterministic. */
+int rr_ensemble_stats_dev_ex(const rr_stats_spec *stats, int32_t n_members, const double *x, int64_t member_stride,
+                             int64_t ld, int64_t rows, int64_t n_out, const int32_t *subset, const double *thr,
+                             int64_t ldt, void *const *out, int64_t ldo, int out_f32, double *peak, int32_t *peak_row,
+                             int64_t ldk, int64_t row0, void *stream);
 
 /* rr_route_ensemble_host with the member outputs reduced on the device: per time chunk, all members are routed into an
  * fp64 device scratch, averaged over `resample` rows, reduced to the statistics of `stats`, and only those are copied
@@ -226,6 +245,16 @@ int rr_route_ensemble_stats_host(rr_plan *p, int mode, const double *q_init, int
                                  const void *const *lateral, int lateral_f32, int64_t ldl, const rr_stats_spec *stats,
                                  void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq, double *q_mean,
                                  int64_t T, int64_t substeps, int64_t resample);
+
+/* rr_route_ensemble_stats_host with the plan's thresholds (rr_plan_set_thresholds; RR_STAT_EXCEED reads the threshold
+ * of reach subset[c] for column c) and optional horizon peaks: peak / peak_row are host [n_stats][ldk], fp64 value and
+ * int32 output row relative to this call, over the call's T / resample rows (the library initialises them).  out may be
+ * NULL when peak is given: then no per-step rows are kept on the device or copied back. */
+int rr_route_ensemble_stats_host_ex(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
+                                    const void *const *lateral, int lateral_f32, int64_t ldl, const rr_stats_spec *stats,
+                                    void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq,
+                                    double *q_mean, int64_t T, int64_t substeps, int64_t resample, double *peak,
+                                    int32_t *peak_row, int64_t ldk);
 
 /* Kernel launches issued by this library on this thread since the last reset (bench.py's
  * gpu_launches claim). */

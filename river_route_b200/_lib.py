@@ -82,6 +82,12 @@ def _load() -> C.CDLL:
         'rr_route_ensemble_stats_host': (C.c_int, [vp, C.c_int, f64p, i64, i32, C.POINTER(vp), C.c_int, i64,
                                                    C.POINTER(StatsSpec), C.POINTER(vp), i64, C.c_int, f64p, i64, f64p, i64,
                                                    i64, i64]),
+        'rr_plan_set_thresholds': (C.c_int, [vp, i32, f64p, i64]),
+        'rr_ensemble_stats_dev_ex': (C.c_int, [C.POINTER(StatsSpec), i32, vp, i64, i64, i64, i64, vp, vp, i64, C.POINTER(vp),
+                                               i64, C.c_int, vp, vp, i64, i64, vp]),
+        'rr_route_ensemble_stats_host_ex': (C.c_int, [vp, C.c_int, f64p, i64, i32, C.POINTER(vp), C.c_int, i64,
+                                                      C.POINTER(StatsSpec), C.POINTER(vp), i64, C.c_int, f64p, i64, f64p,
+                                                      i64, i64, i64, f64p, c_i32p, i64]),
         'rr_launch_count': (i64, [C.c_int]),
         'rr_timing_enable': (C.c_int, [C.c_int]),
         'rr_timing_read': (C.c_int, [f64p, c_i64p, C.c_int]),
@@ -112,7 +118,8 @@ EXPORTED_SYMBOLS = (
     'rr_plan_create', 'rr_plan_destroy', 'rr_plan_get_info', 'rr_plan_set_coefficients', 'rr_route_dev',
     'rr_route_host', 'rr_plan_set_output_subset', 'rr_route_host_ex', 'rr_route_host_typed', 'rr_transform_create', 'rr_transform_set_uh', 'rr_transform_get_uh_state',
     'rr_transform_destroy', 'rr_runoff_route_host', 'rr_route_ensemble_dev', 'rr_route_ensemble_host', 'rr_plan_tile_rows',
-    'rr_ensemble_stats_dev', 'rr_route_ensemble_stats_host', 'rr_launch_count', 'rr_timing_enable', 'rr_timing_read', 'rr_uh_convolve_dev', 'rr_uh_convolve_host',
+    'rr_ensemble_stats_dev', 'rr_route_ensemble_stats_host', 'rr_plan_set_thresholds', 'rr_ensemble_stats_dev_ex',
+    'rr_route_ensemble_stats_host_ex', 'rr_launch_count', 'rr_timing_enable', 'rr_timing_read', 'rr_uh_convolve_dev', 'rr_uh_convolve_host',
     'rr_weights_transform_dev', 'rr_weights_transform_host', 'rr_plan_read_profile', 'rr_host_alloc', 'rr_host_free', 'rr_synth_forest',
     'rr_plan_get_arrays', 'rr_plan_schedule',
 )

@@ -132,6 +132,10 @@ struct rr_device_state {
     double *d_q = nullptr, *d_qfull = nullptr;
     double *ens_q = nullptr;                                                   // ensemble calls: [q_init][mean][member states]
     size_t ens_q_cap = 0;
+    void *ens_peak = nullptr;                                                  // ensemble statistics: running peaks, [S][ld] fp64 | [S][ld] int32
+    size_t ens_peak_cap = 0;
+    double *thr = nullptr;                                                     // device copy of rr_plan::thr
+    uint64_t thr_version = 0;
     // renumbered plans: user -> working index and scratch in the working order
     int32_t *inv = nullptr;
     double *p_lat = nullptr, *p_out = nullptr, *p_q = nullptr;
@@ -213,7 +217,7 @@ void rr_device_release(rr_plan *p) {
     void *ptrs[] = {d->up_ptr, d->up_idx, d->slot_src, d->export_id, d->dep_ptr, d->dep_idx, d->down, d->exp_ro, d->edge_ro,
                     d->skew, d->meta, d->narrow_blocks, d->coef, d->raw, d->done, d->ticket, d->prof,
                     d->s_inb[0], d->s_inb[1], d->s_outb[0], d->s_outb[1], d->s_lat, d->s_conv, d->s_route, d->d_q, d->d_qfull,
-                    d->inv, d->p_lat, d->p_out, d->p_q, d->out_subset, d->ens_q};
+                    d->inv, d->p_lat, d->p_out, d->p_q, d->out_subset, d->ens_q, d->ens_peak, d->thr};
     for (void *q : ptrs)
         if (q) cudaFree(q);
     for (auto &k : d->keys) if (k.dev) cudaFree(k.dev);
@@ -934,6 +938,21 @@ static int upload_subset(rr_plan *p) {
     return 0;
 }
 
+// Device copy of the plan's thresholds, refreshed when rr_plan_set_thresholds changed them.
+static int upload_thresholds(rr_plan *p) {
+    rr_device_state *d = p->dev;
+    if (d->thr_version == p->thr_version) return 0;
+    CK(cudaDeviceSynchronize());
+    if (d->thr) CK(cudaFree(d->thr));
+    d->thr = nullptr;
+    if (!p->thr.empty()) {
+        CK(cudaMalloc((void **)&d->thr, p->thr.size() * sizeof(double)));
+        CK(cudaMemcpy(d->thr, p->thr.data(), p->thr.size() * sizeof(double), cudaMemcpyHostToDevice));
+    }
+    d->thr_version = p->thr_version;
+    return 0;
+}
+
 // Host arrays: stream time chunks through two device buffers per direction.
 //   s_in : H2D of chunk c+1        (cudaMemcpy2DAsync, pinned source gives full PCIe rate)
 //   s_comp: [weights -> unit hydrograph ->] route chunk c [-> resample / float32]   (state carried on the device)
@@ -1180,7 +1199,9 @@ static int stream_route(rr_plan *p, int mode, double *q_state, double *q_full, c
 // single-member stream (H2D of chunk c+1 | device work of chunk c | D2H of chunk c-1).  The member states stay on the
 // device between chunks; at the end they are copied back and averaged in member order (:145-146).
 // With `stats`, the members' fp64 rows stay on the device and only their statistics (rr_stats.cu) are copied back:
-// out[s] / ldo / out_f32 then describe the statistic arrays, over the plan's output subset.
+// out[s] / ldo / out_f32 then describe the statistic arrays, over the plan's output subset.  With `peak`, the running
+// peaks of every statistic stay on the device for the whole call (-inf at the start, one D2H at the end); out may then
+// be NULL, and no per-step rows are kept or copied.
 // ---------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) member_mean_kernel(const double *__restrict__ states, int64_t ld, int n_members, int64_t n,
                                                            double *__restrict__ mean) {
@@ -1193,8 +1214,9 @@ __global__ void __launch_bounds__(256) member_mean_kernel(const double *__restri
 
 static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int M, const void *const *lateral, int lat_f32,
                               int64_t ldl, void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq,
-                              double *q_mean, int64_t T, int64_t K, int64_t resample, const rr_stats_plan *stats = nullptr) {
-    if (!p || !q_init || !out || M < 1 || M > RR_MAX_MEMBERS) { rr_set_error("bad ensemble arguments (1..64 members)"); return 100; }
+                              double *q_mean, int64_t T, int64_t K, int64_t resample, const rr_stats_plan *stats = nullptr,
+                              double *peak = nullptr, int32_t *peak_row = nullptr, int64_t ldk = 0) {
+    if (!p || !q_init || !(out || (stats && peak)) || M < 1 || M > RR_MAX_MEMBERS) { rr_set_error("bad ensemble arguments (1..64 members)"); return 100; }
     if (mode == RR_MODE_UNIT) { rr_set_error("ensemble calls support Muskingum / RapidMuskingum"); return 100; }
     const bool has_lat = mode != RR_MODE_MUSKINGUM;
     if (has_lat && !lateral) { rr_set_error("null argument"); return 100; }
@@ -1207,8 +1229,8 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
     const int64_t n = p->n, ldd = ((n + 31) / 32) * 32;
     const int64_t n_out = (stats && !p->out_subset.empty()) ? (int64_t)p->out_subset.size() : n;   // columns copied back
     const int64_t ldd_out = ((n_out + 31) / 32) * 32;
-    const int n_arrays = stats ? stats->n_stats : M;                                                 // host arrays per row
-    if (ldo < n_out || (has_lat && ldl < n) || (q_final && ldq < n) || (ld_init != 0 && ld_init < n)) { rr_set_error("leading dimension smaller than n"); return 100; }
+    const int n_arrays = !out ? 0 : stats ? stats->n_stats : M;                                      // host arrays per row
+    if ((out && ldo < n_out) || (peak && ldk < n_out) || (has_lat && ldl < n) || (q_final && ldq < n) || (ld_init != 0 && ld_init < n)) { rr_set_error("leading dimension smaller than n"); return 100; }
     const bool pipe = pipeline_ok(p, mode, K);
     const bool fused = pipe && resample == 1 && !stats;
     const bool cast_first = has_lat && lat_f32 && !(pipe && K == 1);
@@ -1226,15 +1248,17 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         const double ldp = (double)(((p->n_work + 31) / 32) * 32), md = (double)M * (double)ldd;
         const double caps[] = {(double)d->s_inb_cap[0], (double)d->s_inb_cap[1], (double)d->s_outb_cap[0], (double)d->s_outb_cap[1],
                                (double)d->s_lat_cap, (double)d->s_route_cap, 8.0 * d->p_lat_cap, 8.0 * d->p_out_cap,
-                               8.0 * d->p_q_cap, (double)d->ens_q_cap};
+                               8.0 * d->p_q_cap, (double)d->ens_q_cap, (double)d->ens_peak_cap, 0.0};
         auto extra = [&](int64_t c) {
             const double tiles = (double)M * ldp * 8.0 * (double)((c + RR_FLAG_ROWS - 1) / RR_FLAG_ROWS * RR_FLAG_ROWS);
-            const double outb = (double)stats->n_stats * (double)(c / resample) * (double)ldd_out * (double)es_out;
+            const double outb = out ? (double)stats->n_stats * (double)(c / resample) * (double)ldd_out * (double)es_out : 0.0;
+            // the last two: running peaks (12 B per statistic and column), thresholds still to upload
             const double need[] = {has_lat ? md * c * es_in : 0.0, has_lat ? md * c * es_in : 0.0, outb, outb,
                                    cast_first ? md * c * 8.0 : 0.0, md * c * 8.0, has_lat ? tiles : 0.0, tiles,
-                                   4.0 * M * ldp * 8.0, (M + 2.0) * ldd * 8.0};
+                                   4.0 * M * ldp * 8.0, (M + 2.0) * ldd * 8.0, peak ? 12.0 * stats->n_stats * ldd_out : 0.0,
+                                   stats->exceed && d->thr_version != p->thr_version ? 8.0 * (double)p->n_thr * (double)n : 0.0};
             double more = 0.0;
-            for (int b = 0; b < 10; ++b) more += std::max(0.0, need[b] - caps[b]);
+            for (int b = 0; b < 12; ++b) more += std::max(0.0, need[b] - caps[b]);
             return more;
         };
         const double room = 0.92 * (double)free_b - (double)(256ll << 20);
@@ -1270,9 +1294,21 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
     const size_t in_member = (size_t)chunk * ldd * es_in, out_member = (size_t)rows_out_max * ldd_out * es_out;
     for (int k = 0; k < 2; ++k) {
         if (has_lat && (rc = grow_bytes(&d->s_inb[k], &d->s_inb_cap[k], in_member * M))) return rc;
-        if ((rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], out_member * n_arrays))) return rc;
+        if (n_arrays && (rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], out_member * n_arrays))) return rc;
     }
     if (stats && (rc = upload_subset(p))) return rc;
+    if (stats && stats->exceed && (rc = upload_thresholds(p))) return rc;
+    rr_stats_ext ex;
+    if (stats) {
+        ex.thr = stats->exceed ? d->thr : nullptr;
+        ex.ldt = n;
+        if (peak) {
+            if ((rc = grow_bytes(&d->ens_peak, &d->ens_peak_cap, (size_t)12 * stats->n_stats * ldd_out))) return rc;
+            ex.peak = (double *)d->ens_peak;
+            ex.peak_row = (int32_t *)(ex.peak + (size_t)stats->n_stats * ldd_out);
+            ex.ldk = ldd_out;
+        }
+    }
     const size_t f64_member = (size_t)chunk * ldd * 8;
     if (cast_first && (rc = grow_bytes((void **)&d->s_lat, &d->s_lat_cap, f64_member * M))) return rc;
     if (!fused && (rc = grow_bytes((void **)&d->s_route, &d->s_route_cap, f64_member * M))) return rc;
@@ -1282,6 +1318,7 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
     const bool shared_init = ld_init == 0;
     if (shared_init) CK(cudaMemcpyAsync(d_q0, q_init, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, d->s_comp));
     else CK(cudaMemcpy2DAsync(d_qm, (size_t)ldd * 8, q_init, (size_t)ld_init * 8, (size_t)n * 8, M, cudaMemcpyHostToDevice, d->s_comp));
+    if (ex.peak && (rc = rr_stats_peak_init(ex.peak, ex.peak_row, (int64_t)stats->n_stats * ldd_out, d->s_comp))) return rc;
     const int64_t n_chunks = (T + chunk - 1) / chunk;
     auto copy_in = [&](int64_t c) -> int {
         if (!has_lat) return 0;
@@ -1327,8 +1364,10 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
             void *dst[RR_MAX_STATS];
             for (int s = 0; s < stats->n_stats; ++s) dst[s] = (char *)d->s_outb[k] + out_member * s;
             rr_timer tm(3, d->s_comp);
+            ex.row0 = c * chunk / resample;
             rc = rr_stats_launch(*stats, d->s_route, (int64_t)(f64_member / 8), ldd, (int)resample, rows_out, n_out,
-                                 p->out_subset.empty() ? nullptr : d->out_subset, dst, ldd_out, out_f32, d->s_comp);
+                                 p->out_subset.empty() ? nullptr : d->out_subset, out ? dst : nullptr, ldd_out, out_f32, ex,
+                                 d->s_comp);
             if (rc) return rc;
         } else if (!fused) {
             for (int m = 0; m < M; ++m) {
@@ -1355,6 +1394,12 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         CK(cudaMemcpyAsync(q_mean, d_mean, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
     }
     if (q_final) CK(cudaMemcpy2DAsync(q_final, (size_t)ldq * 8, d_qm, (size_t)ldd * 8, (size_t)n * 8, M, cudaMemcpyDeviceToHost, d->s_comp));
+    if (ex.peak) {
+        CK(cudaMemcpy2DAsync(peak, (size_t)ldk * 8, ex.peak, (size_t)ldd_out * 8, (size_t)n_out * 8, stats->n_stats,
+                             cudaMemcpyDeviceToHost, d->s_comp));
+        CK(cudaMemcpy2DAsync(peak_row, (size_t)ldk * 4, ex.peak_row, (size_t)ldd_out * 4, (size_t)n_out * 4, stats->n_stats,
+                             cudaMemcpyDeviceToHost, d->s_comp));
+    }
     CK(cudaStreamSynchronize(d->s_comp));
     CK(cudaStreamSynchronize(d->s_out));
     CK(cudaStreamSynchronize(d->s_in));
@@ -1372,17 +1417,29 @@ static int ensemble_settle(rr_plan *p, int rc) {
     return rc;
 }
 
+extern "C" int rr_route_ensemble_stats_host_ex(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
+                                               const void *const *lateral, int lateral_f32, int64_t ldl, const rr_stats_spec *stats,
+                                               void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq,
+                                               double *q_mean, int64_t T, int64_t substeps, int64_t resample, double *peak,
+                                               int32_t *peak_row, int64_t ldk) {
+    rr_stats_plan sp;
+    int rc = rr_stats_prepare(stats, n_members, p ? p->n_thr : 0, &sp);
+    if (rc) return rc;
+    if (!out && !peak) { rr_set_error("no output: give per-step arrays (out), peaks (peak / peak_row) or both"); return 100; }
+    if (peak && !peak_row) { rr_set_error("peak needs peak_row"); return 100; }
+    for (int s = 0; out && s < sp.n_stats; ++s)
+        if (!out[s]) { rr_set_error("null output array"); return 100; }
+    return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
+                                                 q_final, ldq, q_mean, T, substeps, resample, &sp, peak, peak_row, ldk));
+}
+
 extern "C" int rr_route_ensemble_stats_host(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
                                             const void *const *lateral, int lateral_f32, int64_t ldl, const rr_stats_spec *stats,
                                             void *const *out, int64_t ldo, int out_f32, double *q_final, int64_t ldq,
                                             double *q_mean, int64_t T, int64_t substeps, int64_t resample) {
-    rr_stats_plan sp;
-    int rc = rr_stats_prepare(stats, n_members, &sp);
-    if (rc) return rc;
-    for (int s = 0; out && s < sp.n_stats; ++s)
-        if (!out[s]) { rr_set_error("null output array"); return 100; }
-    return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
-                                                 q_final, ldq, q_mean, T, substeps, resample, &sp));
+    if (!out) { rr_set_error("bad ensemble arguments (1..64 members)"); return 100; }
+    return rr_route_ensemble_stats_host_ex(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, stats, out, ldo, out_f32,
+                                           q_final, ldq, q_mean, T, substeps, resample, nullptr, nullptr, 0);
 }
 
 extern "C" int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
@@ -1391,6 +1448,17 @@ extern "C" int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init
                                       int64_t resample) {
     return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
                                                  q_final, ldq, q_mean, T, substeps, resample));
+}
+
+extern "C" int rr_plan_set_thresholds(rr_plan *p, int32_t n_thr, const double *thr, int64_t ldt) {
+    if (!p || n_thr < 0 || (n_thr > 0 && (!thr || ldt < p->n))) { rr_set_error("bad argument"); return 100; }
+    p->thr.resize((size_t)n_thr * (size_t)p->n);
+    for (int32_t r = 0; r < n_thr; ++r)
+        std::copy(thr + (size_t)r * ldt, thr + (size_t)r * ldt + p->n, p->thr.begin() + (size_t)r * p->n);
+    if (n_thr == 0) p->thr.shrink_to_fit();
+    p->n_thr = n_thr;
+    p->thr_version++;
+    return 0;
 }
 
 extern "C" int rr_plan_set_output_subset(rr_plan *p, int64_t n_sub, const int32_t *idx) {

@@ -60,6 +60,9 @@ struct rr_plan {
     uint64_t coeff_version = 0;
     std::vector<int32_t> out_subset;   // river segments (user indices) the host streaming calls copy back; empty = all
     uint64_t out_subset_version = 0;
+    std::vector<double> thr;           // [n_thr][n] per-river thresholds (user order) of RR_STAT_EXCEED; uploaded lazily
+    int64_t n_thr = 0;
+    uint64_t thr_version = 0;
     rr_device_state *dev = nullptr;
 };
 
@@ -91,11 +94,24 @@ void rr_device_release(rr_plan *p);  // frees p->dev (rr_api.cu)
 
 // rr_stats.cu: a validated rr_stats_spec with the percentile positions resolved for M members
 struct rr_stats_plan {
-    int32_t n_stats = 0, n_members = 0, sort = 0;
-    int32_t kind[RR_MAX_STATS] = {}, lo[RR_MAX_STATS] = {}, hi[RR_MAX_STATS] = {};
+    int32_t n_stats = 0, n_members = 0, sort = 0, exceed = 0;
+    int32_t kind[RR_MAX_STATS] = {}, lo[RR_MAX_STATS] = {}, hi[RR_MAX_STATS] = {};   // exceed: lo = threshold row
     double g[RR_MAX_STATS] = {};
 };
-int rr_stats_prepare(const rr_stats_spec *spec, int32_t n_members, rr_stats_plan *out);
-// out[s] + t * ldo + c = statistic s of row t: the members' rows t*k .. t*k+k-1 averaged first (k = resample)
+// n_thr: threshold rows the exceed entries may index (0: none)
+int rr_stats_prepare(const rr_stats_spec *spec, int32_t n_members, int64_t n_thr, rr_stats_plan *out);
+// thresholds and running peaks of one launch (rr_ensemble_stats_dev_ex); all NULL: per-step rows only
+struct rr_stats_ext {
+    const double *thr = nullptr;       // [n_thr][ldt] by reach
+    int64_t ldt = 0;
+    double *peak = nullptr;            // [n_stats][ldk], read and updated
+    int32_t *peak_row = nullptr;
+    int64_t ldk = 0, row0 = 0;         // row0: global row of the launch's first output row
+};
+// out[s] + t * ldo + c = statistic s of row t: the members' rows t*k .. t*k+k-1 averaged first (k = resample); out NULL
+// (or out[s] NULL): no per-step rows
 int rr_stats_launch(const rr_stats_plan &sp, const double *x, int64_t member_stride, int64_t ld, int k, int64_t rows_out,
-                    int64_t n_out, const int32_t *subset, void *const *out, int64_t ldo, int out_f32, void *stream);
+                    int64_t n_out, const int32_t *subset, void *const *out, int64_t ldo, int out_f32, const rr_stats_ext &ex,
+                    void *stream);
+// peak[0 .. count) = -inf, peak_row[0 .. count) = 0
+int rr_stats_peak_init(double *peak, int32_t *peak_row, int64_t count, void *stream);

@@ -16,6 +16,7 @@ from ._lib import lib, check
 
 MODE_MUSKINGUM, MODE_RAPID, MODE_UNIT = 0, 1, 2
 _STAT_KINDS = {'mean': 0, 'std': 1, 'min': 2, 'max': 3}   # RR_STAT_*; 'pQ' is RR_STAT_PERCENTILE (4) with q = Q
+STAT_EXCEED = 5   # RR_STAT_EXCEED: 'exceed_<label>', q = the label's threshold row
 
 
 def downstream_index(river_ids, downstream_ids) -> np.ndarray:
@@ -55,12 +56,17 @@ def label_basins(down: np.ndarray, n_parts: int = 0):
     return basin, int(nb.value), part
 
 
-def parse_statistics(names) -> list:
+def parse_statistics(names, thresholds=()) -> list:
     """
     Ensemble statistic names -> ``[(name, kind, q)]``: ``'mean'``, ``'std'`` (population, ddof=0), ``'min'``, ``'max'``
-    and percentiles ``'p0'`` .. ``'p100'`` (integer q, numpy's default 'linear' method).  At most 16, no duplicates;
-    anything else raises ``ValueError``.
+    and percentiles ``'p0'`` .. ``'p100'`` (integer q, numpy's default 'linear' method).  With threshold labels
+    (``thresholds``, in threshold-row order, e.g. ``('rp2', 'rp10')``), ``'exceed_<label>'`` is the fraction of members
+    strictly above that threshold, ``np.mean(x > thr, axis=0)``, and resolves to ``(name, 5, row of the label)``.  At
+    most 16, no duplicates; anything else raises ``ValueError``.
     """
+    labels = list(thresholds)
+    if len(set(labels)) != len(labels):
+        raise ValueError(f'duplicate threshold labels in {labels}')
     if isinstance(names, str):
         names = [names]
     names = list(names)
@@ -74,16 +80,19 @@ def parse_statistics(names) -> list:
             out.append((name, _STAT_KINDS[name], 0))
         elif name[:1] == 'p' and name[1:].isdigit() and str(int(name[1:])) == name[1:] and int(name[1:]) <= 100:
             out.append((name, 4, int(name[1:])))
+        elif name.startswith('exceed_') and name[7:] in labels:
+            out.append((name, STAT_EXCEED, labels.index(name[7:])))
         else:
-            raise ValueError(f"unknown ensemble statistic {name!r}: use 'mean', 'std', 'min', 'max' or 'p0' .. 'p100'")
+            hint = f", or 'exceed_<label>' with a label of {labels}" if labels else ''
+            raise ValueError(f"unknown ensemble statistic {name!r}: use 'mean', 'std', 'min', 'max' or 'p0' .. 'p100'{hint}")
     if len({o[0] for o in out}) != len(out):
         raise ValueError(f'duplicate ensemble statistics in {names}')
     return out
 
 
-def _stats_spec(names):
+def _stats_spec(names, thresholds=()):
     spec = _lib.StatsSpec()
-    parsed = parse_statistics(names)
+    parsed = parse_statistics(names, thresholds)
     spec.n_stats = len(parsed)
     for s, (_, kind, q) in enumerate(parsed):
         spec.kind[s], spec.q[s] = kind, q
@@ -91,17 +100,31 @@ def _stats_spec(names):
 
 
 def ensemble_stats_dev(stats, n_members: int, x_ptr: int, member_stride: int, ld: int, rows: int, n_out: int,
-                       out_ptrs, ldo: int, out_f32: bool, subset_ptr: int = 0, stream: int = 0) -> None:
+                       out_ptrs, ldo: int, out_f32: bool, subset_ptr: int = 0, stream: int = 0, *, thresholds=(),
+                       thr_ptr: int = 0, ldt: int = 0, peak_ptrs=None, ldk: int = 0, row0: int = 0) -> None:
     """The statistics kernel alone on device pointers (``rr_ensemble_stats_dev``): member m, row t, reach i is
     ``x[m * member_stride + t * ld + i]``; ``out_ptrs[s]`` is (rows, ldo) float32 / float64 of statistic ``stats[s]``;
-    column c shows reach ``subset[c]`` (int32 device array) or reach c.  Asynchronous on ``stream``."""
-    spec = _stats_spec(stats)
-    if len(out_ptrs) != spec.n_stats:
+    column c shows reach ``subset[c]`` (int32 device array) or reach c.  Asynchronous on ``stream``.
+
+    Keyword-only (``rr_ensemble_stats_dev_ex``): ``'exceed_<label>'`` names resolve against ``thresholds`` (labels in
+    row order) and read the fp64 device array ``thr_ptr`` [rows][ldt] at reach ``subset[c]``; ``peak_ptrs = (peak,
+    peak_row)`` are device (S, ldk) float64 / int32 running peaks, updated where a row's value is strictly greater, with
+    rows numbered from ``row0`` (start peak at -inf).  ``out_ptrs`` may be ``None`` when ``peak_ptrs`` is given."""
+    spec = _stats_spec(stats, thresholds)
+    if out_ptrs is not None and len(out_ptrs) != spec.n_stats:
         raise ValueError('one output array per statistic')
     arr = C.c_void_p * spec.n_stats
-    check(lib.rr_ensemble_stats_dev(C.byref(spec), int(n_members), C.c_void_p(x_ptr), int(member_stride), int(ld), int(rows),
-                                    int(n_out), C.c_void_p(subset_ptr or None), arr(*out_ptrs), int(ldo), int(bool(out_f32)),
-                                    C.c_void_p(stream or None)))
+    outs = arr(*out_ptrs) if out_ptrs is not None else None
+    if not (thr_ptr or peak_ptrs is not None or out_ptrs is None):
+        check(lib.rr_ensemble_stats_dev(C.byref(spec), int(n_members), C.c_void_p(x_ptr), int(member_stride), int(ld),
+                                        int(rows), int(n_out), C.c_void_p(subset_ptr or None), outs, int(ldo),
+                                        int(bool(out_f32)), C.c_void_p(stream or None)))
+        return
+    peak, peak_row = peak_ptrs if peak_ptrs is not None else (0, 0)
+    check(lib.rr_ensemble_stats_dev_ex(C.byref(spec), int(n_members), C.c_void_p(x_ptr), int(member_stride), int(ld),
+                                       int(rows), int(n_out), C.c_void_p(subset_ptr or None), C.c_void_p(thr_ptr or None),
+                                       int(ldt), outs, int(ldo), int(bool(out_f32)), C.c_void_p(peak or None),
+                                       C.c_void_p(peak_row or None), int(ldk), int(row0), C.c_void_p(stream or None)))
 
 
 def down_from_csc(indptr, indices, n: int) -> np.ndarray:
@@ -139,6 +162,7 @@ class Plan:
         self._h = handle
         self._coeff_key = None
         self.n_out = self.n                     # columns the host streaming calls copy back (see set_output_subset)
+        self.threshold_labels = ()              # labels of the rows set by set_thresholds
 
     def close(self):
         if getattr(self, '_h', None):
@@ -177,6 +201,25 @@ class Plan:
             raise ValueError('indices must be a 1D list of river segment indices')
         check(lib.rr_plan_set_output_subset(self._h, idx.shape[0], _lib.as_i32p(idx) if idx.shape[0] else None))
         self.n_out = int(idx.shape[0]) or self.n
+
+    def set_thresholds(self, thresholds=None):
+        """
+        Per-river thresholds for the ``'exceed_<label>'`` ensemble statistics: an ordered mapping from label to a float
+        (n,) array in params-file order (e.g. return-period flows; NaN: never exceeded).  The labels are kept in
+        ``threshold_labels``; ``None`` or an empty mapping clears them.
+        """
+        items = list((thresholds or {}).items())
+        labels = tuple(k for k, _ in items)
+        if not all(isinstance(k, str) and k for k in labels) or len(set(labels)) != len(labels):
+            raise ValueError(f'threshold labels must be distinct non-empty strings, got {list(labels)}')
+        rows = np.empty((len(items), self.n), dtype=np.float64)
+        for r, (label, a) in enumerate(items):
+            a = np.asarray(a)
+            if a.shape != (self.n,) or a.dtype.kind != 'f':
+                raise ValueError(f'threshold {label!r} must be a float ({self.n},) array, got {a.dtype} {a.shape}')
+            rows[r] = a
+        check(lib.rr_plan_set_thresholds(self._h, len(items), _lib.as_f64p(rows) if items else None, self.n))
+        self.threshold_labels = labels
 
     # ---- host arrays (numpy) : H2D / route / D2H streamed inside the library ----
     def route_host(self, mode: int, q_state: np.ndarray, lateral, out: np.ndarray, substeps: int, q_full=None,
@@ -318,34 +361,43 @@ class Plan:
         return q_mean
 
     def route_ensemble_stats_host(self, mode: int, q_init: np.ndarray, laterals, stats, outs, substeps: int,
-                                  resample: int = 1, q_final: np.ndarray | None = None):
+                                  resample: int = 1, q_final: np.ndarray | None = None, peaks=None):
         """
         As ``route_ensemble_host`` -- same members, inputs, state chaining, ``q_final`` and returned member-mean state --
         but the members' discharge stays on the device: per time chunk it is averaged over ``resample`` rows and reduced
-        to the statistics named in ``stats`` (see ``parse_statistics``), and only those cross PCIe.  ``outs[s]`` is
-        (T / resample, n_out) float32 or float64 (all the same dtype) for statistic ``stats[s]``; n_out follows the
-        output subset (``set_output_subset``).  Every statistic equals numpy on the stacked fp64 member outputs bit for
-        bit (``np.mean`` / ``np.std`` / ``np.min`` / ``np.max`` / ``np.percentile`` over axis 0).
+        to the statistics named in ``stats`` (see ``parse_statistics``; ``'exceed_<label>'`` against the labels of
+        ``set_thresholds``), and only those cross PCIe.  ``outs[s]`` is (T / resample, n_out) float32 or float64 (all
+        the same dtype) for statistic ``stats[s]``; n_out follows the output subset (``set_output_subset``).  Every
+        statistic equals numpy on the stacked fp64 member outputs bit for bit (``np.mean`` / ``np.std`` / ``np.min`` /
+        ``np.max`` / ``np.percentile`` over axis 0; exceedance ``np.mean(x > thr, axis=0)``).
+
+        ``peaks = (values, rows)``, (S, n_out) float64 and int32 arrays, receives each statistic's maximum over this
+        call's output rows and the first row where it occurs (``rows.max(axis=0)`` / ``rows.argmax(axis=0)`` of the fp64
+        statistic rows), kept on the device for the whole call.  ``outs`` may then be ``None``: no per-step rows are
+        kept or copied back, and T comes from the lateral arrays.
         """
-        spec = _stats_spec(stats)
+        spec = _stats_spec(stats, self.threshold_labels)
         M = len(laterals) if laterals is not None else 0
         if mode == MODE_MUSKINGUM:
             raise ValueError('ensemble statistics need lateral inflows (RapidMuskingum members)')
         if not 1 <= M <= 64:
             raise ValueError('ensemble statistics need 1 to 64 members')
-        if len(outs) != spec.n_stats:
+        if outs is None and peaks is None:
+            raise ValueError('give per-step arrays (outs), peaks or both')
+        if outs is not None and len(outs) != spec.n_stats:
             raise ValueError('one output array per statistic')
         if q_init.dtype != np.float64 or not q_init.flags.c_contiguous or q_init.shape not in ((self.n,), (M, self.n)):
             raise ValueError('q_init must be a contiguous float64 (n,) vector or (members, n) array')
         ld_init = self.n if q_init.ndim == 2 else 0
         resample = int(resample)
         n_out = self.n_out
-        T = outs[0].shape[0] * resample
-        odt = outs[0].dtype
-        for o in outs:
-            if o.dtype != odt or odt not in (np.float64, np.float32) or o.shape != (T // resample, n_out) or \
-                    _lib.rows_ld(o) != _lib.rows_ld(outs[0]):
-                raise ValueError('statistic arrays must share dtype (float64 / float32), shape (T / resample, n_out) and row stride')
+        T = outs[0].shape[0] * resample if outs is not None else laterals[0].shape[0]
+        if outs is not None:
+            odt = outs[0].dtype
+            for o in outs:
+                if o.dtype != odt or odt not in (np.float64, np.float32) or o.shape != (T // resample, n_out) or \
+                        _lib.rows_ld(o) != _lib.rows_ld(outs[0]):
+                    raise ValueError('statistic arrays must share dtype (float64 / float32), shape (T / resample, n_out) and row stride')
         ldt = laterals[0].dtype
         for a in laterals:
             if a.dtype != ldt or ldt not in (np.float64, np.float32) or a.shape != (T, self.n) or \
@@ -353,13 +405,21 @@ class Plan:
                 raise ValueError('lateral arrays must share dtype (float64 / float32), shape (T, n) and row stride')
         if q_final is not None and (q_final.dtype != np.float64 or q_final.shape != (M, self.n) or not q_final.flags.c_contiguous):
             raise ValueError('q_final must be a contiguous float64 (members, n) array')
+        if peaks is not None:
+            pv, pr = peaks
+            if pv.dtype != np.float64 or pr.dtype != np.int32 or pv.shape != (spec.n_stats, n_out) or \
+                    pr.shape != pv.shape or not (pv.flags.c_contiguous and pr.flags.c_contiguous):
+                raise ValueError('peaks must be contiguous (S, n_out) float64 values and int32 rows')
         q_mean = np.empty(self.n, dtype=np.float64)
         arr_m, arr_s = C.c_void_p * M, C.c_void_p * spec.n_stats
-        check(lib.rr_route_ensemble_stats_host(
+        check(lib.rr_route_ensemble_stats_host_ex(
             self._h, int(mode), _lib.as_f64p(q_init), ld_init, M, arr_m(*[a.ctypes.data for a in laterals]),
-            int(ldt == np.float32), _lib.rows_ld(laterals[0]), C.byref(spec), arr_s(*[o.ctypes.data for o in outs]),
-            _lib.rows_ld(outs[0]), int(odt == np.float32), _lib.as_f64p(q_final) if q_final is not None else None, self.n,
-            _lib.as_f64p(q_mean), T, int(substeps), resample))
+            int(ldt == np.float32), _lib.rows_ld(laterals[0]), C.byref(spec),
+            arr_s(*[o.ctypes.data for o in outs]) if outs is not None else None,
+            _lib.rows_ld(outs[0]) if outs is not None else 0, int(outs is not None and odt == np.float32),
+            _lib.as_f64p(q_final) if q_final is not None else None, self.n, _lib.as_f64p(q_mean), T, int(substeps), resample,
+            _lib.as_f64p(pv) if peaks is not None else None, _lib.as_i32p(pr) if peaks is not None else None,
+            n_out if peaks is not None else 0))
         return q_mean
 
     def tile_rows(self, T: int, substeps: int = 1) -> int:

@@ -18,7 +18,7 @@ from typing import Any, Callable, Iterator
 import numpy as np
 import pandas as pd
 
-from .plan import MODE_MUSKINGUM, MODE_RAPID, MODE_UNIT, Plan, downstream_index, parse_statistics
+from .plan import MODE_MUSKINGUM, MODE_RAPID, MODE_UNIT, STAT_EXCEED, Plan, downstream_index, parse_statistics
 from .runoff import runoff_to_qlateral
 from .uhkernels import UnitHydrograph
 
@@ -383,12 +383,12 @@ class Muskingum:
         with self._open_discharge_file(dates, q_array.shape[1], q_file, routed_file) as out:
             out.write_rows(0, q_array)
 
-    def _open_discharge_file(self, dates, n_cols, q_file, routed_file='', statistics=None):
+    def _open_discharge_file(self, dates, n_cols, q_file, routed_file='', statistics=None, horizon='steps'):
         """The same file, opened for writing row slabs as they come back from the GPU (streamed runs)."""
         ids = getattr(self, 'river_ids_all', self.river_ids) if getattr(self, '_output_idx', None) is None \
             else self.river_ids[self._output_idx]
         return _DischargeFile(q_file, dates, ids, n_cols, self.cfg.var_river_id, self.cfg.var_discharge, routed_file,
-                              statistics)
+                              statistics, horizon)
 
 
 class TransformMuskingum(Muskingum):
@@ -398,7 +398,8 @@ class TransformMuskingum(Muskingum):
     _mode = MODE_RAPID
     _ensemble_stats = None
 
-    def set_ensemble_statistics(self, path, statistics=('mean', 'std', 'min', 'max', 'p25', 'p50', 'p75')):
+    def set_ensemble_statistics(self, path, statistics=('mean', 'std', 'min', 'max', 'p25', 'p50', 'p75'),
+                                thresholds=None, horizon='steps'):
         """
         Extension: in ``runoff_processing_mode='ensemble'`` with ``qlateral_files``, write per-time-step statistics
         across the members to ONE netCDF at ``path`` instead of one discharge file per member.  The statistics are
@@ -408,9 +409,53 @@ class TransformMuskingum(Muskingum):
         attribute).  ``statistics``: ``'mean'``, ``'std'`` (ddof=0), ``'min'``, ``'max'``, ``'p0'`` .. ``'p100'``; each
         equals numpy's over the members' fp64 discharge, cast to float32.  The final channel state is the member mean,
         as without statistics.  ``path=None`` switches back to member files.
+
+        Flood warnings: ``thresholds`` is a table (a parquet path or a DataFrame) with a river-id column
+        (``cfg.var_river_id``) and one column of per-river flows per label, e.g. return periods ``rp2`` .. ``rp100``.
+        ``'exceed_<label>'`` is then the fraction of members whose discharge is strictly above the river's threshold,
+        ``np.mean(x > thr, axis=0)``, written as ``<var_discharge>_exceed_<label>`` (units ``1``, attribute
+        ``threshold``).  Rivers missing from the table get NaN thresholds, which are never exceeded (0); table rivers
+        outside the network are ignored; duplicate ids, or no id of the network in the table, raise ``ValueError``.
+
+        ``horizon``: ``'steps'`` writes the per-step variables; ``'peaks'`` writes, per statistic, its maximum over the
+        whole forecast horizon, ``<var_discharge>_<stat>_peak(river_id)`` (float32 of the fp64 peak), and the time of
+        its first occurrence, ``<var_discharge>_<stat>_peak_time(river_id)`` (seconds since the first output time),
+        and no per-step variables: no per-step rows are copied back from the device; ``'both'`` writes both.  The peak
+        time is the first argmax of the fp64 statistic, so it can differ from the argmax of the float32 per-step
+        variable where two fp64 values round to the same float32.
         """
-        self._ensemble_stats = None if path is None else (str(path), parse_statistics(statistics))
+        if horizon not in ('steps', 'peaks', 'both'):
+            raise ValueError(f"horizon must be 'steps', 'peaks' or 'both', got {horizon!r}")
+        if path is None:
+            self._ensemble_stats = None
+            return self
+        table, labels = None, ()
+        if thresholds is not None:
+            table = thresholds if isinstance(thresholds, pd.DataFrame) else pd.read_parquet(thresholds)
+            if self.cfg.var_river_id not in table.columns:
+                raise ValueError(f'thresholds table needs a {self.cfg.var_river_id!r} column')
+            labels = tuple(str(c) for c in table.columns if c != self.cfg.var_river_id)
+        self._ensemble_stats = (str(path), parse_statistics(statistics, labels), table, horizon)
         return self
+
+    def _threshold_rows(self, table, labels):
+        """The thresholds table's columns ``labels`` on the params-file river order: {label: (n,) float64}, NaN for
+        rivers the table does not list."""
+        rid = self.cfg.var_river_id
+        ids = table[rid].to_numpy(dtype=np.int64)
+        if np.unique(ids).shape[0] != ids.shape[0]:
+            raise ValueError('thresholds table lists a river id more than once')
+        pos = pd.Index(ids).get_indexer(self.river_ids)
+        hit = pos >= 0
+        if not hit.any():
+            raise ValueError(f'no river id of the thresholds table is in the network ({rid!r})')
+        cols = {str(c): c for c in table.columns if c != rid}
+        rows = {}
+        for label in labels:
+            col = table[cols[label]].to_numpy(dtype=np.float64)
+            rows[label] = np.full(self.n, np.nan)
+            rows[label][hit] = col[pos[hit]]
+        return rows
 
     def _qlateral_generator(self) -> Iterator[tuple]:
         """Yields (dates, (T, n) fp64 lateral array, input file, output file) per input file (:30-51)."""
@@ -655,11 +700,15 @@ class TransformMuskingum(Muskingum):
         RR_ROUTER_SLAB_BYTES over all members; reads and writes run on the thread pool around the device call.
         """
         from concurrent.futures import ThreadPoolExecutor
-        path, parsed = self._ensemble_stats
+        path, parsed, table, horizon = self._ensemble_stats
         cfg = self.cfg
         M = len(cfg.qlateral_files)
         names = [p[0] for p in parsed]
         n, S = self.n, len(parsed)
+        steps, want_peaks = horizon != 'peaks', horizon != 'steps'
+        used = list(dict.fromkeys(p[0][7:] for p in parsed if p[1] == STAT_EXCEED))   # labels, in order of first use
+        if used:
+            self.plan.set_thresholds(self._threshold_rows(table, used))
         srcs = []
         try:
             for lat_file in cfg.qlateral_files:
@@ -682,11 +731,17 @@ class TransformMuskingum(Muskingum):
             slab = min(T, max(unit, rows // unit * unit))
             starts = list(range(0, T, slab))
             lat = [[self._pinned(('elat', b, m), (slab, n), dtype) for m in range(M)] for b in range(2)]
-            out = [[self._pinned(('estat', b, s), (slab // k, self._n_out), np.float32) for s in range(S)] for b in range(2)]
+            out = [[self._pinned(('estat', b, s), (slab // k, self._n_out), np.float32) for s in range(S)] for b in range(2)] \
+                if steps else None
+            if want_peaks:
+                # per-call peaks, merged over the slabs on the host with the same strict '>' (the earliest row wins)
+                call_peak = (np.empty((S, self._n_out)), np.empty((S, self._n_out), dtype=np.int32))
+                peak, peak_row = np.full((S, self._n_out), -np.inf), np.zeros((S, self._n_out), dtype=np.int64)
             states = np.empty((M, n), dtype=np.float64)
             q_members = self.channel_state.astype(np.float64, copy=True)
             out_file = self._open_discharge_file(dates[::k] if k > 1 else dates, self._n_out, path,
-                                                 ', '.join(str(f) for f in cfg.qlateral_files), statistics=parsed)
+                                                 ', '.join(str(f) for f in cfg.qlateral_files), statistics=parsed,
+                                                 horizon=horizon)
             with out_file, ThreadPoolExecutor(max_workers=4) as pool:
                 def read(s_):
                     t0, t1 = starts[s_], min(T, starts[s_] + slab)
@@ -704,16 +759,28 @@ class TransformMuskingum(Muskingum):
                         nxt = pool.submit(read, s_ + 1)
                     if pending[s_ % 2] is not None:
                         pending[s_ % 2].result()
-                    out_s = [a[:rows // k] for a in out[s_ % 2]]
+                    out_s = [a[:rows // k] for a in out[s_ % 2]] if steps else None
                     # later slabs start from the members' own states (q_members is states once the first slab is done)
-                    mean = self.plan.route_ensemble_stats_host(self._mode, q_members, [a[:rows] for a in lat[s_ % 2]], names,
-                                                               out_s, self.num_routing_steps_per_runoff, resample=k,
-                                                               q_final=states)
+                    lat_s = [a[:rows] for a in lat[s_ % 2]]
+                    if want_peaks:
+                        mean = self.plan.route_ensemble_stats_host(self._mode, q_members, lat_s, names, out_s,
+                                                                   self.num_routing_steps_per_runoff, resample=k,
+                                                                   q_final=states, peaks=call_peak)
+                        better = call_peak[0] > peak
+                        np.copyto(peak, call_peak[0], where=better)
+                        np.copyto(peak_row, call_peak[1] + starts[s_] // k, where=better)
+                    else:
+                        mean = self.plan.route_ensemble_stats_host(self._mode, q_members, lat_s, names, out_s,
+                                                                   self.num_routing_steps_per_runoff, resample=k,
+                                                                   q_final=states)
                     q_members = states
-                    pending[s_ % 2] = pool.submit(write, starts[s_] // k, out_s)
+                    if steps:
+                        pending[s_ % 2] = pool.submit(write, starts[s_] // k, out_s)
                 for f in pending:
                     if f is not None:
                         f.result()
+                if want_peaks:
+                    out_file.write_peaks(peak, peak_row)
         finally:
             for src in srcs:
                 src.close()
@@ -1025,9 +1092,11 @@ class UnitMuskingum(TransformMuskingum):
 class _DischargeFile:
     """Discharge netCDF with the reference's layout (Muskingum.py:337-351), written in row slabs."""
 
-    def __init__(self, path, dates, river_ids, n_cols, var_river_id, var_discharge, routed_file='', statistics=None):
+    def __init__(self, path, dates, river_ids, n_cols, var_river_id, var_discharge, routed_file='', statistics=None,
+                 horizon='steps'):
         """``statistics`` (``[(name, kind, q)]`` of ``plan.parse_statistics``): one variable ``<var_discharge>_<name>``
-        per ensemble statistic instead of the one discharge variable."""
+        per ensemble statistic instead of the one discharge variable.  ``horizon`` ('steps' / 'peaks' / 'both', see
+        ``set_ensemble_statistics``): per-step variables, horizon-peak variables (``write_peaks``) or both."""
         from . import ncio
         self.ds = ncio.open_nc(path, 'w')
         ds = self.ds
@@ -1039,21 +1108,46 @@ class _DischargeFile:
         tv[:] = (dates - dates[0]).astype('timedelta64[s]').astype(np.int64)
         iv = ds.createVariable(var_river_id, 'i4', (var_river_id,))
         iv[:] = np.asarray(river_ids).astype(np.int32)
-        self.vars = []
+        self.vars, self.peak_vars = [], []
+        self.dates = dates
         for name, kind, q in statistics or [(None, None, None)]:
-            qv = ds.createVariable(var_discharge if name is None else f'{var_discharge}_{name}', 'f4', ('time', var_river_id))
-            qv.long_name = 'Discharge at catchment outlet' if name is None else \
-                f'Ensemble {name} of the discharge at catchment outlet'
-            qv.standard_name = 'discharge'
-            qv.aggregation_method = 'mean'
-            qv.units = 'm3 s-1'
-            if kind == 4:
-                qv.percentile = q
-            self.vars.append(qv)
-        self.qv = self.vars[0]
+            if horizon != 'peaks':
+                qv = ds.createVariable(var_discharge if name is None else f'{var_discharge}_{name}', 'f4', ('time', var_river_id))
+                self._describe(qv, name, kind, q)
+                self.vars.append(qv)
+            if horizon != 'steps':
+                pv = ds.createVariable(f'{var_discharge}_{name}_peak', 'f4', (var_river_id,))
+                self._describe(pv, name, kind, q)
+                pv.long_name = f'Peak over the forecast horizon of the {pv.long_name[0].lower()}{pv.long_name[1:]}'
+                tv_ = ds.createVariable(f'{var_discharge}_{name}_peak_time', 'f8', (var_river_id,))
+                tv_.long_name = f'Time of the first occurrence of the peak of {var_discharge}_{name}'
+                tv_.units = tv.units
+                self.peak_vars.append((pv, tv_))
+        self.qv = self.vars[0] if self.vars else None
+
+    @staticmethod
+    def _describe(v, name, kind, q):
+        if kind == STAT_EXCEED:
+            v.long_name = f'Fraction of ensemble members above the {name[7:]} threshold'
+            v.units = '1'
+            v.threshold = name[7:]
+            return
+        v.long_name = 'Discharge at catchment outlet' if name is None else f'Ensemble {name} of the discharge at catchment outlet'
+        v.standard_name = 'discharge'
+        v.aggregation_method = 'mean'
+        v.units = 'm3 s-1'
+        if kind == 4:
+            v.percentile = q
 
     def write_rows(self, t0, rows, var=0):
         self.vars[var][t0:t0 + rows.shape[0], :] = rows
+
+    def write_peaks(self, values, rows):
+        """values (S, n_cols) fp64 and rows (S, n_cols) output-row indices: the peak variables of every statistic."""
+        seconds = (self.dates - self.dates[0]).astype('timedelta64[s]').astype(np.float64)
+        for (pv, tv_), v, r in zip(self.peak_vars, values, rows):
+            pv[:] = v.astype(np.float32)
+            tv_[:] = seconds[r]
 
     def close(self):
         if self.ds is not None:
