@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <functional>
 #include <string>
 #include <thread>
 #include <vector>
@@ -115,7 +116,7 @@ struct rr_device_state {
     double *raw = nullptr;
     size_t raw_bytes = 0;
     int32_t *done = nullptr;
-    size_t done_cap = 0;
+    size_t done_bytes = 0;
     unsigned long long *ticket = nullptr, *prof = nullptr;
     int occ[3] = {0, 0, 0}, occ_direct[3] = {0, 0, 0};
     // host streaming path
@@ -139,7 +140,7 @@ struct rr_device_state {
     // renumbered plans: user -> working index and scratch in the working order
     int32_t *inv = nullptr;
     double *p_lat = nullptr, *p_out = nullptr, *p_q = nullptr;
-    size_t p_lat_cap = 0, p_out_cap = 0, p_q_cap = 0;
+    size_t p_lat_cap = 0, p_out_cap = 0, p_q_cap = 0;   // bytes
     size_t bytes = 0;
 };
 
@@ -149,6 +150,28 @@ static int upload(T **dst, const std::vector<T> &src, size_t &bytes) {
     CK(cudaMalloc((void **)dst, nb));
     if (!src.empty()) CK(cudaMemcpy(*dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice));
     bytes += nb;
+    return 0;
+}
+
+// Device / pinned host buffers that only grow (`cap` and `need` in bytes); growing waits for the device first, since
+// earlier work may still use the old buffer.
+static int grow_device(void **buf, size_t *cap, size_t need, bool zero = false) {
+    if (need <= *cap) return 0;
+    CK(cudaDeviceSynchronize());
+    if (*buf) CK(cudaFree(*buf));
+    *buf = nullptr; *cap = 0;
+    CK(cudaMalloc(buf, need));
+    if (zero) CK(cudaMemset(*buf, 0, need));
+    *cap = need;
+    return 0;
+}
+static int grow_pinned(void **buf, size_t *cap, size_t need) {
+    if (need <= *cap) return 0;
+    CK(cudaDeviceSynchronize());
+    if (*buf) CK(cudaFreeHost(*buf));
+    *buf = nullptr; *cap = 0;
+    CK(cudaHostAlloc(buf, need, cudaHostAllocDefault));
+    *cap = need;
     return 0;
 }
 
@@ -353,21 +376,9 @@ static int launch_route(rr_plan *p, int mode, int n_members, const double *q_ini
     // direct exchange needs no rings: the working discharge array is the exchange buffer
     const size_t raw_need = direct ? (size_t)pitch * sizeof(double)
                                    : ((size_t)n_members * (size_t)d->sched.raw_rows + 1) * pitch * sizeof(double);
-    if (raw_need > d->raw_bytes) {
-        CK(cudaDeviceSynchronize());
-        if (d->raw) CK(cudaFree(d->raw));
-        d->raw = nullptr; d->raw_bytes = 0;
-        CK(cudaMalloc((void **)&d->raw, raw_need));
-        d->raw_bytes = raw_need;
-    }
+    if ((rc = grow_device((void **)&d->raw, &d->raw_bytes, raw_need))) return rc;
     const size_t done_need = (size_t)n_members * p->n_blocks;
-    if (done_need > d->done_cap) {
-        CK(cudaDeviceSynchronize());
-        if (d->done) CK(cudaFree(d->done));
-        d->done = nullptr; d->done_cap = 0;
-        CK(cudaMalloc((void **)&d->done, done_need * sizeof(int32_t)));
-        d->done_cap = done_need;
-    }
+    if ((rc = grow_device((void **)&d->done, &d->done_bytes, done_need * sizeof(int32_t)))) return rc;
 
     rr_route_params P;
     std::memset(&P, 0, sizeof(P));
@@ -582,17 +593,6 @@ static int permute(bool to_working, const double *src, int64_t lds, double *dst,
     rr_count_launch(1);
     return 0;
 }
-static int grow(double **buf, size_t *cap, size_t need) {
-    if (need <= *cap) return 0;
-    CK(cudaDeviceSynchronize());
-    if (*buf) CK(cudaFree(*buf));
-    *buf = nullptr; *cap = 0;
-    CK(cudaMalloc((void **)buf, need * sizeof(double)));
-    CK(cudaMemset(*buf, 0, need * sizeof(double)));   // padding slots of level-sorted plans are routed along: keep them finite
-    *cap = need;
-    return 0;
-}
-
 // Where a call's discharge goes when the caller wants the router loop's tail fused into the last device pass:
 // float32 cast (TransformMuskingum.py:146) and / or an output subset, written straight from the working tiles.
 struct rr_out_spec {
@@ -657,11 +657,12 @@ static int route_any(rr_plan *p, int mode, int n_members, const double *q_init, 
     const int64_t n_tiles = tiled ? (T + trows - 1) / trows : 0;
     const size_t member_elems = tiled ? (size_t)n_tiles * p->n_blocks * tpitch * RR_BLOCK : (size_t)T * ldp;
     const size_t lat_elems = (pipeline && K > 1) ? (size_t)n_tiles * p->n_blocks * lpitch * RR_BLOCK : member_elems;
-    if (has_lat && (rc = grow(&d->p_lat, &d->p_lat_cap, (size_t)n_members * lat_elems + 64))) return rc;
-    if ((rc = grow(&d->p_out, &d->p_out_cap, (size_t)n_members * member_elems + 64))) return rc;
+    // zero-filled: padding slots of level-sorted plans are routed along, keep them finite
+    if (has_lat && (rc = grow_device((void **)&d->p_lat, &d->p_lat_cap, 8 * ((size_t)n_members * lat_elems + 64), true))) return rc;
+    if ((rc = grow_device((void **)&d->p_out, &d->p_out_cap, 8 * ((size_t)n_members * member_elems + 64), true))) return rc;
     // state scratch: [start-of-call state: one shared, or one per member on continued calls][member states][member q_full]
     //                [start-of-call q_full of continued UnitMuskingum pipeline calls]
-    if ((rc = grow(&d->p_q, &d->p_q_cap, (size_t)(4 * n_members) * ldp))) return rc;
+    if ((rc = grow_device((void **)&d->p_q, &d->p_q_cap, 8 * (size_t)(4 * n_members) * ldp, true))) return rc;
     double *w_init = d->p_q;
     double *wf_init = d->p_q + (size_t)(3 * n_members) * ldp;
     const int64_t init_stride = (direct && !first_call) ? ldp : 0;
@@ -843,23 +844,51 @@ extern "C" int rr_transform_get_uh_state(rr_transform *t, double *state, int64_t
 // Output tail of TransformMuskingum._execute_routing on the device: mean over `k` consecutive rows
 // (reshape(T/k, k, n).mean(axis=1): rows added one after the other, then divided by k; TransformMuskingum.py:128-139)
 // and the cast to float32 the writer receives (:146 / Muskingum.py:259, round to nearest even like numpy's astype).
+// Both kernels stride over rows by gridDim.y (at most 65535), so a chunk may hold any number of rows.
 template <typename OT>
 __global__ void __launch_bounds__(256) finish_output(const double *__restrict__ src, int64_t lds, OT *__restrict__ dst,
-                                                     int64_t ldd, int64_t n_out, int k, const int32_t *__restrict__ subset) {
+                                                     int64_t ldd, int64_t n_out, int64_t rows_out, int k,
+                                                     const int32_t *__restrict__ subset) {
     const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= n_out) return;
     const int64_t i = subset ? (int64_t)__ldg(subset + s) : s;      // output column s shows river segment i
-    const double *p = src + (int64_t)blockIdx.y * k * lds + i;
-    double acc = __ldg(p);
-    for (int r = 1; r < k; ++r) acc += __ldg(p + (int64_t)r * lds);
-    if (k > 1) acc = acc / (double)k;
-    dst[(int64_t)blockIdx.y * ldd + s] = (OT)acc;
+    for (int64_t t = blockIdx.y; t < rows_out; t += gridDim.y) {
+        const double *p = src + t * k * lds + i;
+        double acc = __ldg(p);
+        for (int r = 1; r < k; ++r) acc += __ldg(p + (int64_t)r * lds);
+        if (k > 1) acc = acc / (double)k;
+        dst[t * ldd + s] = (OT)acc;
+    }
 }
 
 __global__ void __launch_bounds__(256) upcast_rows(const float *__restrict__ src, int64_t lds, double *__restrict__ dst, int64_t ldd,
-                                                    int64_t n) {
+                                                    int64_t n, int64_t rows) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) dst[(int64_t)blockIdx.y * ldd + i] = (double)__ldg(src + (int64_t)blockIdx.y * lds + i);
+    if (i >= n) return;
+    for (int64_t t = blockIdx.y; t < rows; t += gridDim.y) dst[t * ldd + i] = (double)__ldg(src + t * lds + i);
+}
+
+static dim3 row_grid(int64_t n, int64_t rows) {
+    return dim3((unsigned)((n + 255) / 256), (unsigned)std::min<int64_t>(rows, 65535));
+}
+// rows x n float32 -> fp64 (exact)
+static int launch_upcast(const float *src, int64_t lds, double *dst, int64_t ldd, int64_t n, int64_t rows, cudaStream_t stream) {
+    rr_timer tm(3, stream);
+    upcast_rows<<<row_grid(n, rows), 256, 0, stream>>>(src, lds, dst, ldd, n, rows);
+    CK(cudaGetLastError());
+    rr_count_launch(1);
+    return 0;
+}
+// rows_out rows of n_out columns (subset: their river segments, NULL: the first n_out), each the mean of k source rows
+static int launch_finish(const double *src, int64_t lds, void *dst, int out_f32, int64_t ldd, int64_t n_out, int64_t rows_out,
+                         int k, const int32_t *subset, cudaStream_t stream) {
+    rr_timer tm(3, stream);
+    const dim3 g = row_grid(n_out, rows_out);
+    if (out_f32) finish_output<float><<<g, 256, 0, stream>>>(src, lds, (float *)dst, ldd, n_out, rows_out, k, subset);
+    else finish_output<double><<<g, 256, 0, stream>>>(src, lds, (double *)dst, ldd, n_out, rows_out, k, subset);
+    CK(cudaGetLastError());
+    rr_count_launch(1);
+    return 0;
 }
 
 int rr_weights_run(int64_t n_rivers, int64_t n_points, int64_t T, const int32_t *indptr, const int32_t *indices,
@@ -923,40 +952,134 @@ struct rr_stream_source {
     int64_t ldx = 0;
 };
 
-// Device copy of the plan's output subset, refreshed when rr_plan_set_output_subset changed it.
-static int upload_subset(rr_plan *p) {
-    rr_device_state *d = p->dev;
-    if (d->out_subset_version == p->out_subset_version) return 0;
+// Device copy of a host vector of the plan (output subset, thresholds), refreshed when its version changed.
+template <typename T>
+static int refresh(T **dev, uint64_t *dev_version, const std::vector<T> &host, uint64_t version) {
+    if (*dev_version == version) return 0;
     CK(cudaDeviceSynchronize());
-    if (d->out_subset) CK(cudaFree(d->out_subset));
-    d->out_subset = nullptr;
-    if (!p->out_subset.empty()) {
-        CK(cudaMalloc((void **)&d->out_subset, p->out_subset.size() * sizeof(int32_t)));
-        CK(cudaMemcpy(d->out_subset, p->out_subset.data(), p->out_subset.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    if (*dev) CK(cudaFree(*dev));
+    *dev = nullptr;
+    if (!host.empty()) {
+        CK(cudaMalloc((void **)dev, host.size() * sizeof(T)));
+        CK(cudaMemcpy(*dev, host.data(), host.size() * sizeof(T), cudaMemcpyHostToDevice));
     }
-    d->out_subset_version = p->out_subset_version;
+    *dev_version = version;
     return 0;
 }
 
-// Device copy of the plan's thresholds, refreshed when rr_plan_set_thresholds changed them.
-static int upload_thresholds(rr_plan *p) {
-    rr_device_state *d = p->dev;
-    if (d->thr_version == p->thr_version) return 0;
-    CK(cudaDeviceSynchronize());
-    if (d->thr) CK(cudaFree(d->thr));
-    d->thr = nullptr;
-    if (!p->thr.empty()) {
-        CK(cudaMalloc((void **)&d->thr, p->thr.size() * sizeof(double)));
-        CK(cudaMemcpy(d->thr, p->thr.data(), p->thr.size() * sizeof(double), cudaMemcpyHostToDevice));
-    }
-    d->thr_version = p->thr_version;
-    return 0;
+// Chunk rows of a host call, from the caller's length model (RR_STREAM_CHUNK_ROWS overrides it; tests force many
+// chunks with it): whole 16-row groups when the direct pipeline runs the call, else whole 8-row groups, then whole
+// output rows, at most T.
+static int64_t round_chunk(int64_t chunk, bool pipe, int64_t resample, int64_t T) {
+    if (const char *env = getenv("RR_STREAM_CHUNK_ROWS")) chunk = std::max(1, atoi(env));
+    if (pipe && chunk >= RR_FLAG_ROWS) chunk = chunk / RR_FLAG_ROWS * RR_FLAG_ROWS;
+    else if (chunk >= 8) chunk = chunk / 8 * 8;
+    chunk = std::max<int64_t>(resample, chunk / resample * resample);
+    return std::min<int64_t>(chunk, T);
 }
 
-// Host arrays: stream time chunks through two device buffers per direction.
+// One direction of a host call's chunk copies: n host arrays (0: nothing crosses), `width` bytes of each row, rows
+// `h_pitch` bytes apart.  In a chunk buffer (device, and the pinned bounce buffer) array a starts at a * stride bytes,
+// its rows d_pitch bytes apart.
+struct rr_chunk_io {
+    int n = 0;
+    const void *const *host = nullptr;
+    size_t width = 0, h_pitch = 0, d_pitch = 0, stride = 0;
+    int64_t lead = 0;      // input: rows before its first row a chunk c > 0 carries too (cumulative grids: one)
+    int64_t row_div = 1;   // output: chunk rows per host row (resampling)
+    bool bounce = false;   // pageable host arrays: through the pinned bounce buffers, copied by host threads
+    char *row(int a, int64_t r) const { return (char *)host[a] + (size_t)r * h_pitch; }
+};
+
+// Host arrays: stream the time chunks [start[c], start[c+1]) through two device buffers per direction.
 //   s_in : H2D of chunk c+1        (cudaMemcpy2DAsync, pinned source gives full PCIe rate)
-//   s_comp: [weights -> unit hydrograph ->] route chunk c [-> resample / float32]   (state carried on the device)
+//   s_comp: work(c, k): the device work of chunk c, from s_inb[k] into s_outb[k]
 //   s_out: D2H of chunk c-1
+// finish() enqueues what follows the last chunk (the final states) before the streams are synchronised.
+static int run_chunks(rr_device_state *d, const std::vector<int64_t> &start, const rr_chunk_io &in, const rr_chunk_io &out,
+                      const std::function<int(int64_t, int)> &work, const std::function<int()> &finish) {
+    int rc;
+    for (int k = 0; k < 2; ++k) {
+        if ((rc = grow_device(&d->s_inb[k], &d->s_inb_cap[k], in.n * in.stride))) return rc;
+        if ((rc = grow_device(&d->s_outb[k], &d->s_outb_cap[k], out.n * out.stride))) return rc;
+    }
+    for (int k = 0; k < 2; ++k) {
+        if (in.bounce && (rc = grow_pinned(&d->h_inb[k], &d->h_inb_cap[k], in.n * in.stride))) return rc;
+        if (out.bounce && (rc = grow_pinned(&d->h_outb[k], &d->h_outb_cap[k], out.n * out.stride))) return rc;
+    }
+    const int64_t n_chunks = (int64_t)start.size() - 1;
+    auto copy_in = [&](int64_t c) -> int {
+        if (!in.n) return 0;
+        const int k = (int)(c & 1);
+        const int64_t r0 = start[c] - (c > 0 ? in.lead : 0), rows = start[c + 1] - r0;
+        if (in.bounce) {
+            if (c >= 2) CK(cudaEventSynchronize(d->ev_in[k]));           // H2D of chunk c-2 has left the bounce buffer
+            for (int a = 0; a < in.n; ++a)
+                parallel_copy_2d((char *)d->h_inb[k] + a * in.stride, in.d_pitch, in.row(a, r0), in.h_pitch, in.width, rows);
+        }
+        if (c >= 2) CK(cudaStreamWaitEvent(d->s_in, d->ev_comp[k], 0));  // buffer free once chunk c-2 was routed
+        for (int a = 0; a < in.n; ++a) {
+            const char *h = in.bounce ? (const char *)d->h_inb[k] + a * in.stride : in.row(a, r0);
+            CK(cudaMemcpy2DAsync((char *)d->s_inb[k] + a * in.stride, in.d_pitch, h, in.bounce ? in.d_pitch : in.h_pitch,
+                                 in.width, rows, cudaMemcpyHostToDevice, d->s_in));
+        }
+        CK(cudaEventRecord(d->ev_in[k], d->s_in));
+        return 0;
+    };
+    // pageable output: chunk c leaves its bounce buffer once its D2H has finished
+    auto drain = [&](int64_t c) -> int {
+        if (!out.bounce || c < 0) return 0;
+        const int k = (int)(c & 1);
+        CK(cudaEventSynchronize(d->ev_out[k]));
+        for (int a = 0; a < out.n; ++a)
+            parallel_copy_2d(out.row(a, start[c] / out.row_div), out.h_pitch, (const char *)d->h_outb[k] + a * out.stride,
+                             out.d_pitch, out.width, (start[c + 1] - start[c]) / out.row_div);
+        return 0;
+    };
+    if ((rc = copy_in(0))) return rc;
+    for (int64_t c = 0; c < n_chunks; ++c) {
+        const int k = (int)(c & 1);
+        if (in.n) CK(cudaStreamWaitEvent(d->s_comp, d->ev_in[k], 0));
+        if (c >= 2) CK(cudaStreamWaitEvent(d->s_comp, d->ev_out[k], 0));  // out buffer drained
+        if ((rc = work(c, k))) return rc;
+        CK(cudaEventRecord(d->ev_comp[k], d->s_comp));
+        CK(cudaStreamWaitEvent(d->s_out, d->ev_comp[k], 0));
+        const int64_t rows_out = (start[c + 1] - start[c]) / out.row_div;
+        for (int a = 0; a < out.n; ++a) {
+            const char *b = (const char *)d->s_outb[k] + a * out.stride;
+            if (out.bounce)
+                CK(cudaMemcpyAsync((char *)d->h_outb[k] + a * out.stride, b, (size_t)rows_out * out.d_pitch, cudaMemcpyDeviceToHost, d->s_out));
+            else
+                CK(cudaMemcpy2DAsync(out.row(a, start[c] / out.row_div), out.h_pitch, b, out.d_pitch, out.width, rows_out,
+                                     cudaMemcpyDeviceToHost, d->s_out));
+        }
+        CK(cudaEventRecord(d->ev_out[k], d->s_out));
+        // host work of the neighbouring chunks while the device is busy with this one
+        if (c + 1 < n_chunks && (rc = copy_in(c + 1))) return rc;
+        if ((rc = drain(c - 1))) return rc;
+    }
+    if ((rc = drain(n_chunks - 1))) return rc;
+    if ((rc = finish())) return rc;
+    CK(cudaStreamSynchronize(d->s_comp));
+    CK(cudaStreamSynchronize(d->s_out));
+    CK(cudaStreamSynchronize(d->s_in));
+    return 0;
+}
+
+// A failed host call: copies of earlier chunks may still be reading / writing the caller's arrays, so let them finish
+// before the caller gets control back (and possibly frees the arrays); keep the first error message.
+static int settle(rr_plan *p, int rc) {
+    if (rc && p && p->dev) {
+        const std::string msg = rr_last_error();
+        cudaDeviceSynchronize();
+        cudaGetLastError();
+        rr_set_error(msg);
+    }
+    return rc;
+}
+
+// Single-member host calls: [weights -> unit hydrograph ->] route [-> resample / float32] per chunk, the state carried
+// on the device from chunk to chunk.
 static int stream_route_impl(rr_plan *p, int mode, double *q_state, double *q_full, const rr_stream_source &src, void *out,
                              int64_t ldo, int64_t T, int64_t substeps, int out_f32, int64_t resample) {
     if (!p || !q_state || !out) { rr_set_error("null argument"); return 100; }
@@ -982,13 +1105,13 @@ static int stream_route_impl(rr_plan *p, int mode, double *q_state, double *q_fu
     const int64_t ldd = ((n + 31) / 32) * 32;  // device rows start on 256-byte boundaries
     const bool post = out_f32 || resample > 1 || !p->out_subset.empty();
     const bool uh = grid && mode == RR_MODE_UNIT;
+    const bool pipe = pipeline_ok(p, mode, substeps);
     // Chunk length.  Short chunks keep the fill / drain of the three-stage pipeline small (aim: 1/16 of the call),
     // but every chunk is one wavefront launch whose dependency pipeline has to fill again (~20 us per level of the
     // block DAG): a chunk should last at least 4x that, where a row lasts as long as its slowest stage -- H2D, D2H
     // (~45 GB/s each, concurrently) or the device work (~14 ps per reach-substep).  Calls that copy little back
     // (output subsets) or little in (grids) therefore get long, device-efficient chunks; qlateral-in / all-segments-out
-    // calls get short ones.  Bounded by ~1 GiB per transfer buffer and ~4 GiB of fp64 scratch rows; whole 8-row
-    // groups and whole output rows.
+    // calls get short ones.  Bounded by ~1 GiB per transfer buffer and ~4 GiB of fp64 scratch rows.
     const int64_t row_bytes = ldd * 8;
     const double in_row = !has_lat ? 0.0 : (grid ? (double)src.tf->n_points * (src.x_is_f32 ? 4 : 8) : (double)n * (src.lat_f32 ? 4 : 8));
     const double out_row = (double)n_out * (out_f32 ? 4 : 8) / (double)resample;
@@ -998,60 +1121,37 @@ static int stream_route_impl(rr_plan *p, int mode, double *q_state, double *q_fu
     if (uh) min_rows = std::max<int64_t>(min_rows, src.tf->n_ks);
     const int64_t xfer_cap = std::max<int64_t>(min_rows, (int64_t)((double)(1ll << 30) / std::max({in_row, out_row, 1.0})));
     const int64_t cap_rows = std::max<int64_t>(1, std::min<int64_t>(xfer_cap, (4ll << 30) / row_bytes));
-    int64_t chunk = std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(T / 16, min_rows), cap_rows));
-    if (const char *env = getenv("RR_STREAM_CHUNK_ROWS")) chunk = std::max(1, atoi(env));   // tests: force many chunks
+    const int64_t chunk = round_chunk(std::max<int64_t>(1, std::min<int64_t>(std::max<int64_t>(T / 16, min_rows), cap_rows)), pipe,
+                                      resample, T);
     // fused output tail (cast / subset written straight from the working tiles) when the direct pipeline runs the call
-    const bool fused = post && resample == 1 && pipeline_ok(p, mode, substeps);
-    if (pipeline_ok(p, mode, substeps) && chunk >= RR_FLAG_ROWS) chunk = (chunk / RR_FLAG_ROWS) * RR_FLAG_ROWS;   // whole 16-row groups
-    else if (chunk >= 8) chunk = (chunk / 8) * 8;
-    chunk = std::max<int64_t>(resample, (chunk / resample) * resample);
-    chunk = std::min<int64_t>(chunk, T);
+    const bool fused = post && resample == 1 && pipe;
     const size_t es_in = grid ? (src.x_is_f32 ? 4 : 8) : (src.lat_f32 ? 4 : 8), es_out = out_f32 ? 4 : 8;
     const int64_t ld_in = grid ? ((src.tf->n_points + 31) / 32) * 32 : ldd;
-    const size_t need_in = has_lat ? (size_t)(chunk + (grid ? 1 : 0)) * ld_in * es_in : 0;
     const int64_t ldd_out = ((n_out + 31) / 32) * 32;
-    const size_t need_out = (size_t)(chunk / resample) * ldd_out * es_out;
-    auto grow_bytes = [&](void **buf, size_t *cap, size_t need) -> int {
-        if (need <= *cap) return 0;
-        CK(cudaDeviceSynchronize());
-        if (*buf) CK(cudaFree(*buf));
-        *buf = nullptr; *cap = 0;
-        CK(cudaMalloc(buf, need));
-        *cap = need;
-        return 0;
-    };
-    if ((rc = upload_subset(p))) return rc;
-    for (int k = 0; k < 2; ++k) {
-        if ((rc = grow_bytes(&d->s_inb[k], &d->s_inb_cap[k], need_in))) return rc;
-        if ((rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], need_out))) return rc;
-    }
+    if ((rc = refresh(&d->out_subset, &d->out_subset_version, p->out_subset, p->out_subset_version))) return rc;
     const void *h_src = grid ? src.runoff : (const void *)src.lateral;
     const int in_kind = has_lat ? host_pointer_kind(h_src) : RR_PTR_PINNED, out_kind = host_pointer_kind(out);
     if (in_kind == RR_PTR_DEVICE || out_kind == RR_PTR_DEVICE || host_pointer_kind(q_state) == RR_PTR_DEVICE) {
         rr_set_error("the host entry points take host pointers; use rr_route_dev for device-resident arrays");
         return 100;
     }
-    const bool in_bounce = in_kind == RR_PTR_PAGEABLE, out_bounce = out_kind == RR_PTR_PAGEABLE;
-    auto grow_pinned = [&](void **buf, size_t *cap, size_t need) -> int {
-        if (need <= *cap) return 0;
-        CK(cudaDeviceSynchronize());
-        if (*buf) CK(cudaFreeHost(*buf));
-        *buf = nullptr; *cap = 0;
-        CK(cudaHostAlloc(buf, need, cudaHostAllocDefault));
-        *cap = need;
-        return 0;
-    };
-    for (int k = 0; k < 2; ++k) {
-        if (in_bounce && (rc = grow_pinned(&d->h_inb[k], &d->h_inb_cap[k], need_in))) return rc;
-        if (out_bounce && (rc = grow_pinned(&d->h_outb[k], &d->h_outb_cap[k], need_out))) return rc;
-    }
+    rr_chunk_io in, outs;
+    in.n = has_lat ? 1 : 0; in.host = &h_src; in.bounce = in_kind == RR_PTR_PAGEABLE;
+    in.width = (size_t)(grid ? src.tf->n_points : n) * es_in; in.h_pitch = (size_t)(grid ? src.ldx : src.ldl) * es_in;
+    in.d_pitch = (size_t)ld_in * es_in; in.stride = (size_t)(chunk + (grid ? 1 : 0)) * in.d_pitch;
+    // a cumulative grid chunk starts with the last row of the previous chunk (its aggregate is the value to subtract)
+    in.lead = (grid && src.cumulative) ? 1 : 0;
+    const void *h_out = out;
+    outs.n = 1; outs.host = &h_out; outs.bounce = out_kind == RR_PTR_PAGEABLE; outs.row_div = resample;
+    outs.width = (size_t)n_out * es_out; outs.h_pitch = (size_t)ldo * es_out; outs.d_pitch = (size_t)ldd_out * es_out;
+    outs.stride = (size_t)(chunk / resample) * outs.d_pitch;
     const size_t need_f64 = (size_t)chunk * ldd * 8;
     // float32 lateral inflows: the direct pipeline's staging kernel upcasts them on the fly; other paths get an exact
     // upcast into the fp64 scratch first
-    const bool lat_cast = !grid && has_lat && src.lat_f32 && (!pipeline_ok(p, mode, substeps) || mode == RR_MODE_UNIT || substeps > 1);
-    if ((grid || lat_cast) && (rc = grow_bytes((void **)&d->s_lat, &d->s_lat_cap, need_f64))) return rc;
-    if (uh && (rc = grow_bytes((void **)&d->s_conv, &d->s_conv_cap, need_f64))) return rc;
-    if (post && !fused && (rc = grow_bytes((void **)&d->s_route, &d->s_route_cap, need_f64))) return rc;
+    const bool lat_cast = !grid && has_lat && src.lat_f32 && (!pipe || mode == RR_MODE_UNIT || substeps > 1);
+    if ((grid || lat_cast) && (rc = grow_device((void **)&d->s_lat, &d->s_lat_cap, need_f64))) return rc;
+    if (uh && (rc = grow_device((void **)&d->s_conv, &d->s_conv_cap, need_f64))) return rc;
+    if (post && !fused && (rc = grow_device((void **)&d->s_route, &d->s_route_cap, need_f64))) return rc;
     if (!d->d_q) CK(cudaMalloc((void **)&d->d_q, sizeof(double) * (size_t)n));
     if (mode == RR_MODE_UNIT && !d->d_qfull) CK(cudaMalloc((void **)&d->d_qfull, sizeof(double) * (size_t)n));
     CK(cudaMemcpyAsync(d->d_q, q_state, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, d->s_comp));
@@ -1073,59 +1173,21 @@ static int stream_route_impl(rr_plan *p, int mode, double *q_state, double *q_fu
         start.push_back(T);
     }
     const int64_t n_chunks = (int64_t)start.size() - 1;
-    auto rows_of = [&](int64_t c) { return start[c + 1] - start[c]; };
-    // a cumulative grid chunk starts with the last row of the previous chunk (its aggregate is the value to subtract)
-    auto lead_of = [&](int64_t c) -> int64_t { return (grid && src.cumulative && c > 0) ? 1 : 0; };
-    auto copy_in = [&](int64_t c) -> int {
-        if (!has_lat) return 0;
-        const int k = (int)(c & 1);
-        const int64_t lead = lead_of(c), nrows = rows_of(c) + lead;
-        const size_t width = grid ? (size_t)src.tf->n_points * es_in : (size_t)n * es_in;
-        const size_t h_pitch = grid ? (size_t)src.ldx * es_in : (size_t)src.ldl * es_in, d_pitch = (size_t)ld_in * es_in;
-        const char *h = (const char *)h_src + (size_t)(start[c] - lead) * h_pitch;
-        size_t pitch = h_pitch;
-        if (in_bounce) {
-            if (c >= 2) CK(cudaEventSynchronize(d->ev_in[k]));           // H2D of chunk c-2 has left the bounce buffer
-            parallel_copy_2d((char *)d->h_inb[k], d_pitch, h, h_pitch, width, nrows);
-            h = (const char *)d->h_inb[k];
-            pitch = d_pitch;
-        }
-        if (c >= 2) CK(cudaStreamWaitEvent(d->s_in, d->ev_comp[k], 0));  // buffer free once chunk c-2 was routed
-        CK(cudaMemcpy2DAsync(d->s_inb[k], d_pitch, h, pitch, width, nrows, cudaMemcpyHostToDevice, d->s_in));
-        CK(cudaEventRecord(d->ev_in[k], d->s_in));
-        return 0;
-    };
-    // pageable output: chunk c leaves its bounce buffer once its D2H has finished
-    auto drain = [&](int64_t c) -> int {
-        if (!out_bounce || c < 0) return 0;
-        const int k = (int)(c & 1);
-        CK(cudaEventSynchronize(d->ev_out[k]));
-        parallel_copy_2d((char *)out + (size_t)(start[c] / resample) * ldo * es_out, (size_t)ldo * es_out,
-                         (const char *)d->h_outb[k], (size_t)ldd_out * es_out, (size_t)n_out * es_out, rows_of(c) / resample);
-        return 0;
-    };
-    if ((rc = copy_in(0))) return rc;
-    for (int64_t c = 0; c < n_chunks; ++c) {
-        const int k = (int)(c & 1);
-        const int64_t rows = rows_of(c);
-        if (has_lat) CK(cudaStreamWaitEvent(d->s_comp, d->ev_in[k], 0));
-        if (c >= 2) CK(cudaStreamWaitEvent(d->s_comp, d->ev_out[k], 0));  // out buffer drained
+    const int32_t *sub = p->out_subset.empty() ? nullptr : d->out_subset;
+    auto work = [&](int64_t c, int k) -> int {
+        const int64_t rows = start[c + 1] - start[c], lead = (c > 0) ? in.lead : 0;
         const double *lat = (const double *)d->s_inb[k];
         if (lat_cast) {
-            rr_timer tm(3, d->s_comp);
-            dim3 g((unsigned)((n + 255) / 256), (unsigned)rows);
-            upcast_rows<<<g, 256, 0, d->s_comp>>>((const float *)d->s_inb[k], ld_in, d->s_lat, ldd, n);
-            CK(cudaGetLastError());
-            rr_count_launch(1);
+            if ((rc = launch_upcast((const float *)d->s_inb[k], ld_in, d->s_lat, ldd, n, rows, d->s_comp))) return rc;
             lat = d->s_lat;
         }
         if (grid) {
             const rr_transform *t = src.tf;
             {
                 rr_timer tm(3, d->s_comp);
-                rc = rr_weights_run(n, t->n_points, rows + lead_of(c), t->indptr, t->indices, t->w, d->s_inb[k],
+                rc = rr_weights_run(n, t->n_points, rows + lead, t->indptr, t->indices, t->w, d->s_inb[k],
                                     src.x_is_f32, ld_in, d->s_lat, ldd, src.cumulative, src.force_positive,
-                                    (src.as_volumes && !uh) ? t->area : nullptr, lead_of(c), d->s_comp);
+                                    (src.as_volumes && !uh) ? t->area : nullptr, lead, d->s_comp);
             }
             if (rc) return rc;
             lat = d->s_lat;
@@ -1141,63 +1203,34 @@ static int stream_route_impl(rr_plan *p, int mode, double *q_state, double *q_fu
         const double *lat1[1] = {lat};
         double *out1[1] = {route_out}, *qs1[1] = {d->d_q}, *qf1[1] = {d->d_qfull};
         rr_out_spec spec;
-        spec.dst = d->s_outb[k]; spec.f32 = out_f32; spec.ld = ldd_out; spec.n_out = n_out;
-        spec.subset = p->out_subset.empty() ? nullptr : d->out_subset;
+        spec.dst = d->s_outb[k]; spec.f32 = out_f32; spec.ld = ldd_out; spec.n_out = n_out; spec.subset = sub;
         rc = route_any(p, mode, 1, d->d_q, lat1, ldd, out1, ldd, qs1, qf1, rows, substeps,
                        router_level && c == 0, router_level && c == n_chunks - 1, d->s_comp, fused ? &spec : nullptr,
                        (!grid && has_lat && src.lat_f32 && !lat_cast) ? 1 : 0);
         if (rc) return rc;
-        const int64_t rows_out = rows / resample;
-        if (post && !fused) {
-            rr_timer tm(3, d->s_comp);
-            dim3 g((unsigned)((n_out + 255) / 256), (unsigned)rows_out);
-            const int32_t *sub = p->out_subset.empty() ? nullptr : d->out_subset;
-            if (out_f32) finish_output<float><<<g, 256, 0, d->s_comp>>>(d->s_route, ldd, (float *)d->s_outb[k], ldd_out, n_out, (int)resample, sub);
-            else finish_output<double><<<g, 256, 0, d->s_comp>>>(d->s_route, ldd, (double *)d->s_outb[k], ldd_out, n_out, (int)resample, sub);
-            CK(cudaGetLastError());
-            rr_count_launch(1);
-        }
-        CK(cudaEventRecord(d->ev_comp[k], d->s_comp));
-        CK(cudaStreamWaitEvent(d->s_out, d->ev_comp[k], 0));
-        if (out_bounce)
-            CK(cudaMemcpyAsync(d->h_outb[k], d->s_outb[k], (size_t)rows_out * ldd_out * es_out, cudaMemcpyDeviceToHost, d->s_out));
-        else
-            CK(cudaMemcpy2DAsync((char *)out + (size_t)(start[c] / resample) * ldo * es_out, ldo * es_out, d->s_outb[k],
-                                 ldd_out * es_out, n_out * es_out, rows_out, cudaMemcpyDeviceToHost, d->s_out));
-        CK(cudaEventRecord(d->ev_out[k], d->s_out));
-        // host work of the neighbouring chunks while the device is busy with this one
-        if (c + 1 < n_chunks && (rc = copy_in(c + 1))) return rc;
-        if ((rc = drain(c - 1))) return rc;
-    }
-    if ((rc = drain(n_chunks - 1))) return rc;
-    CK(cudaMemcpyAsync(q_state, d->d_q, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
-    if (!router_level)
-        CK(cudaMemcpyAsync(q_full, d->d_qfull, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
-    CK(cudaStreamSynchronize(d->s_comp));
-    CK(cudaStreamSynchronize(d->s_out));
-    CK(cudaStreamSynchronize(d->s_in));
-    return 0;
+        if (post && !fused)
+            return launch_finish(d->s_route, ldd, d->s_outb[k], out_f32, ldd_out, n_out, rows / resample, (int)resample, sub, d->s_comp);
+        return 0;
+    };
+    auto finish = [&]() -> int {
+        CK(cudaMemcpyAsync(q_state, d->d_q, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
+        if (!router_level)
+            CK(cudaMemcpyAsync(q_full, d->d_qfull, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
+        return 0;
+    };
+    return run_chunks(d, start, in, outs, work, finish);
 }
 
 static int stream_route(rr_plan *p, int mode, double *q_state, double *q_full, const rr_stream_source &src, void *out,
                         int64_t ldo, int64_t T, int64_t substeps, int out_f32, int64_t resample) {
-    const int rc = stream_route_impl(p, mode, q_state, q_full, src, out, ldo, T, substeps, out_f32, resample);
-    if (rc && p && p->dev) {
-        // copies of earlier chunks may still be reading / writing the caller's arrays: let them finish before the
-        // caller gets control back (and possibly frees the arrays); keep the first error message
-        const std::string msg = rr_last_error();
-        cudaDeviceSynchronize();
-        cudaGetLastError();
-        rr_set_error(msg);
-    }
-    return rc;
+    return settle(p, stream_route_impl(p, mode, q_state, q_full, src, out, ldo, T, substeps, out_f32, resample));
 }
 
 // ---------------------------------------------------------------------------------------------------
 // Ensembles from host arrays: the members of one time chunk are routed by ONE wavefront launch (tickets x members),
-// every member from the same initial state (TransformMuskingum.py:121-126); chunks are double-buffered like the
-// single-member stream (H2D of chunk c+1 | device work of chunk c | D2H of chunk c-1).  The member states stay on the
-// device between chunks; at the end they are copied back and averaged in member order (:145-146).
+// every member from the same initial state (TransformMuskingum.py:121-126); chunks go through the same double-buffered
+// pipeline as single-member calls (run_chunks), copied straight from and to the caller's arrays.  The member states
+// stay on the device between chunks; at the end they are copied back and averaged in member order (:145-146).
 // With `stats`, the members' fp64 rows stay on the device and only their statistics (rr_stats.cu) are copied back:
 // out[s] / ldo / out_f32 then describe the statistic arrays, over the plan's output subset.  With `peak`, the running
 // peaks of every statistic stay on the device for the whole call (-inf at the start, one D2H at the end); out may then
@@ -1247,8 +1280,8 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         CK(cudaMemGetInfo(&free_b, &total_b));
         const double ldp = (double)(((p->n_work + 31) / 32) * 32), md = (double)M * (double)ldd;
         const double caps[] = {(double)d->s_inb_cap[0], (double)d->s_inb_cap[1], (double)d->s_outb_cap[0], (double)d->s_outb_cap[1],
-                               (double)d->s_lat_cap, (double)d->s_route_cap, 8.0 * d->p_lat_cap, 8.0 * d->p_out_cap,
-                               8.0 * d->p_q_cap, (double)d->ens_q_cap, (double)d->ens_peak_cap, 0.0};
+                               (double)d->s_lat_cap, (double)d->s_route_cap, (double)d->p_lat_cap, (double)d->p_out_cap,
+                               (double)d->p_q_cap, (double)d->ens_q_cap, (double)d->ens_peak_cap, 0.0};
         auto extra = [&](int64_t c) {
             const double tiles = (double)M * ldp * 8.0 * (double)((c + RR_FLAG_ROWS - 1) / RR_FLAG_ROWS * RR_FLAG_ROWS);
             const double outb = out ? (double)stats->n_stats * (double)(c / resample) * (double)ldd_out * (double)es_out : 0.0;
@@ -1275,85 +1308,59 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         }
         chunk = lo;
     }
-    if (const char *env = getenv("RR_STREAM_CHUNK_ROWS")) chunk = std::max(1, atoi(env));
-    const int64_t unit = pipe ? RR_FLAG_ROWS : 8;
-    if (chunk >= unit) chunk = chunk / unit * unit;
-    chunk = std::max<int64_t>(resample, chunk / resample * resample);
-    chunk = std::min<int64_t>(chunk, T);
-    const int64_t rows_out_max = chunk / resample;
-    auto grow_bytes = [&](void **buf, size_t *cap, size_t need) -> int {
-        if (need <= *cap) return 0;
-        CK(cudaDeviceSynchronize());
-        if (*buf) CK(cudaFree(*buf));
-        *buf = nullptr; *cap = 0;
-        CK(cudaMalloc(buf, need));
-        *cap = need;
-        return 0;
-    };
-    // out_member: one host array's rows of a chunk (a member's discharge, or one statistic)
-    const size_t in_member = (size_t)chunk * ldd * es_in, out_member = (size_t)rows_out_max * ldd_out * es_out;
-    for (int k = 0; k < 2; ++k) {
-        if (has_lat && (rc = grow_bytes(&d->s_inb[k], &d->s_inb_cap[k], in_member * M))) return rc;
-        if (n_arrays && (rc = grow_bytes(&d->s_outb[k], &d->s_outb_cap[k], out_member * n_arrays))) return rc;
-    }
-    if (stats && (rc = upload_subset(p))) return rc;
-    if (stats && stats->exceed && (rc = upload_thresholds(p))) return rc;
+    chunk = round_chunk(chunk, pipe, resample, T);
+    // one host array's rows of a chunk: a member's inflows; a member's discharge, or one statistic
+    rr_chunk_io in, outs;
+    in.n = has_lat ? M : 0; in.host = lateral;
+    in.width = (size_t)n * es_in; in.h_pitch = (size_t)ldl * es_in; in.d_pitch = (size_t)ldd * es_in;
+    in.stride = (size_t)chunk * in.d_pitch;
+    outs.n = n_arrays; outs.host = out; outs.row_div = resample;
+    outs.width = (size_t)n_out * es_out; outs.h_pitch = (size_t)ldo * es_out; outs.d_pitch = (size_t)ldd_out * es_out;
+    outs.stride = (size_t)(chunk / resample) * outs.d_pitch;
+    if (stats && (rc = refresh(&d->out_subset, &d->out_subset_version, p->out_subset, p->out_subset_version))) return rc;
+    if (stats && stats->exceed && (rc = refresh(&d->thr, &d->thr_version, p->thr, p->thr_version))) return rc;
     rr_stats_ext ex;
     if (stats) {
         ex.thr = stats->exceed ? d->thr : nullptr;
         ex.ldt = n;
         if (peak) {
-            if ((rc = grow_bytes(&d->ens_peak, &d->ens_peak_cap, (size_t)12 * stats->n_stats * ldd_out))) return rc;
+            if ((rc = grow_device(&d->ens_peak, &d->ens_peak_cap, (size_t)12 * stats->n_stats * ldd_out))) return rc;
             ex.peak = (double *)d->ens_peak;
             ex.peak_row = (int32_t *)(ex.peak + (size_t)stats->n_stats * ldd_out);
             ex.ldk = ldd_out;
         }
     }
-    const size_t f64_member = (size_t)chunk * ldd * 8;
-    if (cast_first && (rc = grow_bytes((void **)&d->s_lat, &d->s_lat_cap, f64_member * M))) return rc;
-    if (!fused && (rc = grow_bytes((void **)&d->s_route, &d->s_route_cap, f64_member * M))) return rc;
-    if ((rc = grow_bytes((void **)&d->ens_q, &d->ens_q_cap, (size_t)(M + 2) * ldd * 8))) return rc;
+    const size_t f64_member = (size_t)chunk * ldd;   // elements
+    if (cast_first && (rc = grow_device((void **)&d->s_lat, &d->s_lat_cap, 8 * f64_member * M))) return rc;
+    if (!fused && (rc = grow_device((void **)&d->s_route, &d->s_route_cap, 8 * f64_member * M))) return rc;
+    if ((rc = grow_device((void **)&d->ens_q, &d->ens_q_cap, (size_t)(M + 2) * ldd * 8))) return rc;
     double *d_q0 = d->ens_q, *d_mean = d->ens_q + ldd, *d_qm = d->ens_q + 2 * ldd;
     // shared initial state (a reference call), or one state per member (a later time slab of the same members)
     const bool shared_init = ld_init == 0;
     if (shared_init) CK(cudaMemcpyAsync(d_q0, q_init, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, d->s_comp));
     else CK(cudaMemcpy2DAsync(d_qm, (size_t)ldd * 8, q_init, (size_t)ld_init * 8, (size_t)n * 8, M, cudaMemcpyHostToDevice, d->s_comp));
     if (ex.peak && (rc = rr_stats_peak_init(ex.peak, ex.peak_row, (int64_t)stats->n_stats * ldd_out, d->s_comp))) return rc;
-    const int64_t n_chunks = (T + chunk - 1) / chunk;
-    auto copy_in = [&](int64_t c) -> int {
-        if (!has_lat) return 0;
-        const int k = (int)(c & 1);
-        const int64_t rows = std::min<int64_t>(chunk, T - c * chunk);
-        if (c >= 2) CK(cudaStreamWaitEvent(d->s_in, d->ev_comp[k], 0));
-        for (int m = 0; m < M; ++m)
-            CK(cudaMemcpy2DAsync((char *)d->s_inb[k] + in_member * m, (size_t)ldd * es_in,
-                                 (const char *)lateral[m] + (size_t)(c * chunk) * ldl * es_in, (size_t)ldl * es_in, (size_t)n * es_in,
-                                 rows, cudaMemcpyHostToDevice, d->s_in));
-        CK(cudaEventRecord(d->ev_in[k], d->s_in));
-        return 0;
-    };
-    if ((rc = copy_in(0))) return rc;
-    for (int64_t c = 0; c < n_chunks; ++c) {
-        const int k = (int)(c & 1);
-        const int64_t rows = std::min<int64_t>(chunk, T - c * chunk), rows_out = rows / resample;
-        if (has_lat) CK(cudaStreamWaitEvent(d->s_comp, d->ev_in[k], 0));
-        if (c >= 2) CK(cudaStreamWaitEvent(d->s_comp, d->ev_out[k], 0));
+    std::vector<int64_t> start;
+    for (int64_t at = 0; at < T; at += chunk) start.push_back(at);
+    start.push_back(T);
+    const int64_t n_chunks = (int64_t)start.size() - 1;
+    const int32_t *sub = p->out_subset.empty() ? nullptr : d->out_subset;
+    auto work = [&](int64_t c, int k) -> int {
+        const int64_t rows = start[c + 1] - start[c], rows_out = rows / resample;
         const double *lat_m[RR_MAX_MEMBERS];
         double *out_m[RR_MAX_MEMBERS], *qs_m[RR_MAX_MEMBERS];
         rr_out_spec spec[RR_MAX_MEMBERS];
         for (int m = 0; m < M; ++m) {
-            const char *in = (const char *)d->s_inb[k] + in_member * m;
+            const char *x = (const char *)d->s_inb[k] + in.stride * m;
             if (cast_first) {
-                double *dst = d->s_lat + (f64_member / 8) * m;
-                dim3 g((unsigned)((n + 255) / 256), (unsigned)rows);
-                upcast_rows<<<g, 256, 0, d->s_comp>>>((const float *)in, ldd, dst, ldd, n);
-                rr_count_launch(1);
-                in = (const char *)dst;
+                double *dst = d->s_lat + f64_member * m;
+                if ((rc = launch_upcast((const float *)x, ldd, dst, ldd, n, rows, d->s_comp))) return rc;
+                x = (const char *)dst;
             }
-            lat_m[m] = (const double *)in;
-            out_m[m] = fused ? nullptr : d->s_route + (f64_member / 8) * m;
+            lat_m[m] = (const double *)x;
+            out_m[m] = fused ? nullptr : d->s_route + f64_member * m;
             qs_m[m] = d_qm + (size_t)m * ldd;
-            spec[m].dst = (char *)d->s_outb[k] + out_member * m; spec[m].f32 = out_f32; spec[m].ld = ldd_out;
+            spec[m].dst = (char *)d->s_outb[k] + outs.stride * m; spec[m].f32 = out_f32; spec[m].ld = ldd_out;
             spec[m].subset = nullptr; spec[m].n_out = n;
         }
         rc = route_any(p, mode, M, d_q0, has_lat ? lat_m : nullptr, ldd, out_m, ldd, qs_m, nullptr, rows, K, c == 0 && shared_init, c == n_chunks - 1,
@@ -1362,59 +1369,33 @@ static int ensemble_host_impl(rr_plan *p, int mode, const double *q_init, int64_
         if (stats) {
             // the members' fp64 rows in s_route -> resample -> statistics, one launch
             void *dst[RR_MAX_STATS];
-            for (int s = 0; s < stats->n_stats; ++s) dst[s] = (char *)d->s_outb[k] + out_member * s;
+            for (int s = 0; s < stats->n_stats; ++s) dst[s] = (char *)d->s_outb[k] + outs.stride * s;
             rr_timer tm(3, d->s_comp);
-            ex.row0 = c * chunk / resample;
-            rc = rr_stats_launch(*stats, d->s_route, (int64_t)(f64_member / 8), ldd, (int)resample, rows_out, n_out,
-                                 p->out_subset.empty() ? nullptr : d->out_subset, out ? dst : nullptr, ldd_out, out_f32, ex,
-                                 d->s_comp);
-            if (rc) return rc;
-        } else if (!fused) {
-            for (int m = 0; m < M; ++m) {
-                dim3 g((unsigned)((n + 255) / 256), (unsigned)rows_out);
-                if (out_f32) finish_output<float><<<g, 256, 0, d->s_comp>>>(out_m[m], ldd, (float *)spec[m].dst, ldd, n, (int)resample, nullptr);
-                else finish_output<double><<<g, 256, 0, d->s_comp>>>(out_m[m], ldd, (double *)spec[m].dst, ldd, n, (int)resample, nullptr);
-                rr_count_launch(1);
-            }
-            CK(cudaGetLastError());
+            ex.row0 = start[c] / resample;
+            return rr_stats_launch(*stats, d->s_route, (int64_t)f64_member, ldd, (int)resample, rows_out, n_out, sub,
+                                   out ? dst : nullptr, ldd_out, out_f32, ex, d->s_comp);
         }
-        CK(cudaEventRecord(d->ev_comp[k], d->s_comp));
-        CK(cudaStreamWaitEvent(d->s_out, d->ev_comp[k], 0));
-        for (int a = 0; a < n_arrays; ++a)
-            CK(cudaMemcpy2DAsync((char *)out[a] + (size_t)(c * chunk / resample) * ldo * es_out, (size_t)ldo * es_out,
-                                 (char *)d->s_outb[k] + out_member * a, (size_t)ldd_out * es_out, (size_t)n_out * es_out, rows_out,
-                                 cudaMemcpyDeviceToHost, d->s_out));
-        CK(cudaEventRecord(d->ev_out[k], d->s_out));
-        if (c + 1 < n_chunks && (rc = copy_in(c + 1))) return rc;
-    }
-    if (q_mean) {
-        member_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, d->s_comp>>>(d_qm, ldd, M, n, d_mean);
-        CK(cudaGetLastError());
-        rr_count_launch(1);
-        CK(cudaMemcpyAsync(q_mean, d_mean, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
-    }
-    if (q_final) CK(cudaMemcpy2DAsync(q_final, (size_t)ldq * 8, d_qm, (size_t)ldd * 8, (size_t)n * 8, M, cudaMemcpyDeviceToHost, d->s_comp));
-    if (ex.peak) {
-        CK(cudaMemcpy2DAsync(peak, (size_t)ldk * 8, ex.peak, (size_t)ldd_out * 8, (size_t)n_out * 8, stats->n_stats,
-                             cudaMemcpyDeviceToHost, d->s_comp));
-        CK(cudaMemcpy2DAsync(peak_row, (size_t)ldk * 4, ex.peak_row, (size_t)ldd_out * 4, (size_t)n_out * 4, stats->n_stats,
-                             cudaMemcpyDeviceToHost, d->s_comp));
-    }
-    CK(cudaStreamSynchronize(d->s_comp));
-    CK(cudaStreamSynchronize(d->s_out));
-    CK(cudaStreamSynchronize(d->s_in));
-    return 0;
-}
-
-// failed ensemble calls: earlier chunks' copies may still use the caller's arrays; let them finish, keep the message
-static int ensemble_settle(rr_plan *p, int rc) {
-    if (rc && p && p->dev) {
-        const std::string msg = rr_last_error();
-        cudaDeviceSynchronize();
-        cudaGetLastError();
-        rr_set_error(msg);
-    }
-    return rc;
+        for (int m = 0; !fused && m < M; ++m)
+            if ((rc = launch_finish(out_m[m], ldd, spec[m].dst, out_f32, ldd, n, rows_out, (int)resample, nullptr, d->s_comp))) return rc;
+        return 0;
+    };
+    auto finish = [&]() -> int {
+        if (q_mean) {
+            member_mean_kernel<<<(unsigned)((n + 255) / 256), 256, 0, d->s_comp>>>(d_qm, ldd, M, n, d_mean);
+            CK(cudaGetLastError());
+            rr_count_launch(1);
+            CK(cudaMemcpyAsync(q_mean, d_mean, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, d->s_comp));
+        }
+        if (q_final) CK(cudaMemcpy2DAsync(q_final, (size_t)ldq * 8, d_qm, (size_t)ldd * 8, (size_t)n * 8, M, cudaMemcpyDeviceToHost, d->s_comp));
+        if (ex.peak) {
+            CK(cudaMemcpy2DAsync(peak, (size_t)ldk * 8, ex.peak, (size_t)ldd_out * 8, (size_t)n_out * 8, stats->n_stats,
+                                 cudaMemcpyDeviceToHost, d->s_comp));
+            CK(cudaMemcpy2DAsync(peak_row, (size_t)ldk * 4, ex.peak_row, (size_t)ldd_out * 4, (size_t)n_out * 4, stats->n_stats,
+                                 cudaMemcpyDeviceToHost, d->s_comp));
+        }
+        return 0;
+    };
+    return run_chunks(d, start, in, outs, work, finish);
 }
 
 extern "C" int rr_route_ensemble_stats_host_ex(rr_plan *p, int mode, const double *q_init, int64_t ld_init, int32_t n_members,
@@ -1429,7 +1410,7 @@ extern "C" int rr_route_ensemble_stats_host_ex(rr_plan *p, int mode, const doubl
     if (peak && !peak_row) { rr_set_error("peak needs peak_row"); return 100; }
     for (int s = 0; out && s < sp.n_stats; ++s)
         if (!out[s]) { rr_set_error("null output array"); return 100; }
-    return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
+    return settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
                                                  q_final, ldq, q_mean, T, substeps, resample, &sp, peak, peak_row, ldk));
 }
 
@@ -1446,7 +1427,7 @@ extern "C" int rr_route_ensemble_host(rr_plan *p, int mode, const double *q_init
                                       const void *const *lateral, int lateral_f32, int64_t ldl, void *const *out, int64_t ldo,
                                       int out_f32, double *q_final, int64_t ldq, double *q_mean, int64_t T, int64_t substeps,
                                       int64_t resample) {
-    return ensemble_settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
+    return settle(p, ensemble_host_impl(p, mode, q_init, ld_init, n_members, lateral, lateral_f32, ldl, out, ldo, out_f32,
                                                  q_final, ldq, q_mean, T, substeps, resample));
 }
 

@@ -631,7 +631,7 @@ class TransformMuskingum(Muskingum):
         states = np.empty((M, n), dtype=np.float64)
         budget = float(os.environ.get('RR_ROUTER_SLAB_BYTES', 2 << 30))
         q0 = self.channel_state.astype(np.float64, copy=True)
-        done = 0
+        done, mean = 0, None
         with ThreadPoolExecutor(max_workers=4) as pool:
             while done < M:
                 srcs = [_LateralFile(pairs[done][0])]
@@ -642,45 +642,33 @@ class TransformMuskingum(Muskingum):
                     k = self.num_runoff_steps_per_discharge if self.dt_discharge > self.dt_runoff else 1
                     unit = int(np.lcm(16, k))
                     G = int(max(1, min(M - done, 64, budget // max(1, unit * n * srcs[0].dtype.itemsize))))
-                    for f in range(done + 1, done + G):
-                        srcs.append(_LateralFile(pairs[f][0]))
-                    for src, (lat_file, _) in zip(srcs, pairs[done:done + G]):
-                        self.logger.info(f'Routing qlateral: {lat_file}')
-                        self._check_lateral_shape(src.shape, n)
-                        if src.dates.shape != dates.shape or (len(dates) > 1 and src.dates[1] - src.dates[0] != dates[1] - dates[0]):
-                            raise ValueError('ensemble members must have the same number of time steps and time step')
-                    dtype = srcs[0].dtype if all(s_.dtype == srcs[0].dtype for s_ in srcs) else np.dtype(np.float64)
+                    dtype = self._open_members([p[0] for p in pairs[done:done + G]], srcs)
                     slab = self._slab_rows(T, k, G * n * dtype.itemsize)
                     starts = list(range(0, T, slab))
                     lat = [[self._pinned(('elat', b, m), (slab, n), dtype) for m in range(G)] for b in range(2)]
                     out = [[self._pinned(('eout', b, m), (slab // k, n), np.float32) for m in range(G)] for b in range(2)]
                     files = [self._open_discharge_file(srcs[m].dates[::k] if k > 1 else srcs[m].dates, n, pairs[done + m][1],
                                                        pairs[done + m][0]) for m in range(G)]
+                    q_members = q0
                     try:
                         def read(s_):
                             t0, t1 = starts[s_], min(T, starts[s_] + slab)
                             list(pool.map(lambda m: srcs[m].read(t0, t1, lat[s_ % 2][m]), range(G)))
                             return t1 - t0
-                        nxt = pool.submit(read, 0)
-                        pending = [None, None]
-                        q_members = None
-                        for s_ in range(len(starts)):
-                            rows = nxt.result()
-                            if s_ + 1 < len(starts):
-                                nxt = pool.submit(read, s_ + 1)
-                            if pending[s_ % 2] is not None:
-                                pending[s_ % 2].result()
-                            lat_s = [a[:rows] for a in lat[s_ % 2]]
+
+                        def route(s_, rows):
+                            nonlocal mean, q_members
                             out_s = [a[:rows // k] for a in out[s_ % 2]]
                             group_states = states[done:done + G]
-                            mean = self.plan.route_ensemble_host(self._mode, q0 if q_members is None else q_members, lat_s, out_s,
+                            mean = self.plan.route_ensemble_host(self._mode, q_members, [a[:rows] for a in lat[s_ % 2]], out_s,
                                                                  self.num_routing_steps_per_runoff, resample=k, q_final=group_states)
                             q_members = np.ascontiguousarray(group_states)
-                            r0 = starts[s_] // k
-                            pending[s_ % 2] = pool.submit(lambda r0=r0, out_s=out_s: [f.write_rows(r0, o) for f, o in zip(files, out_s)])
-                        for f in pending:
-                            if f is not None:
-                                f.result()
+                            return out_s
+
+                        def write(s_, out_s):
+                            for f, o in zip(files, out_s):
+                                f.write_rows(starts[s_] // k, o)
+                        self._slab_loop(pool, len(starts), read, route, write)
                     finally:
                         for f in files:
                             f.close()
@@ -707,22 +695,16 @@ class TransformMuskingum(Muskingum):
         n, S = self.n, len(parsed)
         steps, want_peaks = horizon != 'peaks', horizon != 'steps'
         used = list(dict.fromkeys(p[0][7:] for p in parsed if p[1] == STAT_EXCEED))   # labels, in order of first use
+        mean = None
         if used:
             self.plan.set_thresholds(self._threshold_rows(table, used))
-        srcs = []
+        srcs = [_LateralFile(cfg.qlateral_files[0])]
         try:
-            for lat_file in cfg.qlateral_files:
-                srcs.append(_LateralFile(lat_file))
             dates = srcs[0].dates
             self._set_network_and_time_dependent_vectors(dates)
             T = self.num_runoff_steps
             k = self.num_runoff_steps_per_discharge if self.dt_discharge > self.dt_runoff else 1
-            for src, lat_file in zip(srcs, cfg.qlateral_files):
-                self.logger.info(f'Routing qlateral: {lat_file}')
-                self._check_lateral_shape(src.shape, n)
-                if src.dates.shape != dates.shape or (len(dates) > 1 and src.dates[1] - src.dates[0] != dates[1] - dates[0]):
-                    raise ValueError('ensemble members must have the same number of time steps and time step')
-            dtype = srcs[0].dtype if all(s_.dtype == srcs[0].dtype for s_ in srcs) else np.dtype(np.float64)
+            dtype = self._open_members(cfg.qlateral_files, srcs)
             if os.environ.get('RR_ROUTER_SLAB_ROWS'):
                 rows = int(os.environ['RR_ROUTER_SLAB_ROWS'])
             else:
@@ -748,17 +730,8 @@ class TransformMuskingum(Muskingum):
                     list(pool.map(lambda m: srcs[m].read(t0, t1, lat[s_ % 2][m]), range(M)))
                     return t1 - t0
 
-                def write(r0, outs):
-                    for s_, o in enumerate(outs):
-                        out_file.write_rows(r0, o, s_)
-                nxt = pool.submit(read, 0)
-                pending = [None, None]
-                for s_ in range(len(starts)):
-                    rows = nxt.result()
-                    if s_ + 1 < len(starts):
-                        nxt = pool.submit(read, s_ + 1)
-                    if pending[s_ % 2] is not None:
-                        pending[s_ % 2].result()
+                def route(s_, rows):
+                    nonlocal mean, q_members
                     out_s = [a[:rows // k] for a in out[s_ % 2]] if steps else None
                     # later slabs start from the members' own states (q_members is states once the first slab is done)
                     lat_s = [a[:rows] for a in lat[s_ % 2]]
@@ -774,11 +747,12 @@ class TransformMuskingum(Muskingum):
                                                                    self.num_routing_steps_per_runoff, resample=k,
                                                                    q_final=states)
                     q_members = states
-                    if steps:
-                        pending[s_ % 2] = pool.submit(write, starts[s_] // k, out_s)
-                for f in pending:
-                    if f is not None:
-                        f.result()
+                    return out_s
+
+                def write(s_, outs):
+                    for i, o in enumerate(outs):
+                        out_file.write_rows(starts[s_] // k, o, i)
+                self._slab_loop(pool, len(starts), read, route, write if steps else None)
                 if want_peaks:
                     out_file.write_peaks(peak, peak_row)
         finally:
@@ -786,6 +760,43 @@ class TransformMuskingum(Muskingum):
                 src.close()
         self._ensemble_member_states = list(states)
         self.channel_state = mean                      # member-order mean, then / M (TransformMuskingum.py:145-146)
+
+    @staticmethod
+    def _slab_loop(pool, n, read, route, write=None, inline=False):
+        """Slabs 0 .. n-1 with read-ahead and write-behind on ``pool``: ``read(s)`` of slab s+1 runs while slab s is
+        routed by ``route(s, read(s))`` on the calling thread, and ``write(s, route(s, ...))`` of slab s while slab s+1 is
+        routed (``inline``: on the calling thread -- collectives of a sharded run; ``write=None``: nothing to write).
+        Slab s uses the buffers of s % 2: it is routed only after the write of slab s-2 has finished."""
+        nxt = pool.submit(read, 0)
+        pending = [None, None]
+        for s in range(n):
+            got = nxt.result()
+            if s + 1 < n:
+                nxt = pool.submit(read, s + 1)
+            if pending[s % 2] is not None:
+                pending[s % 2].result()                # this output buffer has been written
+            routed = route(s, got)
+            if write is not None and inline:
+                write(s, routed)
+            elif write is not None:
+                pending[s % 2] = pool.submit(write, s, routed)
+        for f in pending:
+            if f is not None:
+                f.result()
+
+    def _open_members(self, lateral_files, srcs):
+        """Open the qlateral files of ensemble members not yet in ``srcs`` (the caller closes them) and check every member
+        against the first: shape (num_runoff_steps, n), the same number of time steps and time step.  Returns the
+        members' common dtype, float64 when they differ."""
+        for lat_file in lateral_files[len(srcs):]:
+            srcs.append(_LateralFile(lat_file))
+        dates = srcs[0].dates
+        for src, lat_file in zip(srcs, lateral_files):
+            self.logger.info(f'Routing qlateral: {lat_file}')
+            self._check_lateral_shape(src.shape, self.n)
+            if src.dates.shape != dates.shape or (len(dates) > 1 and src.dates[1] - src.dates[0] != dates[1] - dates[0]):
+                raise ValueError('ensemble members must have the same number of time steps and time step')
+        return srcs[0].dtype if all(s_.dtype == srcs[0].dtype for s_ in srcs) else np.dtype(np.float64)
 
     def _slab_rows(self, T, k, row_bytes):
         """Rows per slab: about RR_ROUTER_SLAB_BYTES (2 GiB) of lateral inflows, whole 16-row groups of the device
@@ -845,25 +856,14 @@ class TransformMuskingum(Muskingum):
                 out_file.write_rows(r0, rows)
 
         q_t = self.channel_state.astype(np.float64, copy=True)
+
+        def route(s, lat):
+            out = out_bufs[s % 2][:lat.shape[0] // k]
+            self._route_rows(lat, out, k, q_t, s == 0, s == len(starts) - 1)
+            return out
         try:
-            nxt = pool.submit(read, 0)
-            pending = [None, None]
-            for s in range(len(starts)):
-                lat = nxt.result()
-                if s + 1 < len(starts):
-                    nxt = pool.submit(read, s + 1)
-                if pending[s % 2] is not None:
-                    pending[s % 2].result()            # this output buffer has been written
-                out = out_bufs[s % 2][:lat.shape[0] // k]
-                self._route_rows(lat, out, k, q_t, s == 0, s == len(starts) - 1)
-                # collectives of a sharded run stay on the calling thread (one communicator, ordered calls)
-                if sharded:
-                    write(s, out)
-                else:
-                    pending[s % 2] = pool.submit(write, s, out)
-            for f in pending:
-                if f is not None:
-                    f.result()
+            # collectives of a sharded run stay on the calling thread (one communicator, ordered calls)
+            self._slab_loop(pool, len(starts), read, route, write, inline=sharded)
         finally:
             if out_file is not None:
                 out_file.close()
