@@ -516,79 +516,87 @@ __device__ __forceinline__ void st256(double *p, double a, double b, double c, d
 __device__ __forceinline__ void ld256(const double *p, double &a, double &b, double &c, double &d) {
     asm volatile("ld.global.v4.f64 {%0, %1, %2, %3}, [%4];" : "=d"(a), "=d"(b), "=d"(c), "=d"(d) : "l"(p) : "memory");
 }
-template <int ROWS>
+// One group of ROWS rows per grid row; past 65535 groups (the grid.y cap) the STRIDE instantiation strides over them.
+template <int ROWS, bool STRIDE>
 __global__ void __launch_bounds__(256) permute_to_working(const double *__restrict__ src, int64_t lds, double *__restrict__ dst,
                                                           int64_t ldd, const int32_t *__restrict__ inv, int64_t n, int64_t T,
                                                           int64_t tile_rows, int64_t n_blocks, int layout) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int64_t k = __ldg(inv + i);
-    const int64_t t0 = (int64_t)blockIdx.y * ROWS;
-    double v[ROWS];
+    int64_t t0 = (int64_t)blockIdx.y * ROWS;
+    do {
+        double v[ROWS];
 #pragma unroll
-    for (int r = 0; r < ROWS; ++r) v[r] = (t0 + r < T) ? __ldg(src + (t0 + r) * lds + i) : 0.0;
-    if (layout == 2 && (tile_rows % ROWS) == 0) {
-        // the ROWS rows of this reach are contiguous in its tile: whole-sector (ROWS = 16: whole-line) stores
-        double *q = dst + working_index(t0, k, ldd, tile_rows, n_blocks, 2);
+        for (int r = 0; r < ROWS; ++r) v[r] = (t0 + r < T) ? __ldg(src + (t0 + r) * lds + i) : 0.0;
+        if (layout == 2 && (tile_rows % ROWS) == 0) {
+            // the ROWS rows of this reach are contiguous in its tile: whole-sector (ROWS = 16: whole-line) stores
+            double *q = dst + working_index(t0, k, ldd, tile_rows, n_blocks, 2);
 #pragma unroll
-        for (int r = 0; r < ROWS; r += 4) st256(q + r, v[r], v[r + 1], v[r + 2], v[r + 3]);
-        return;
-    }
-    if (layout == 3 && (tile_rows % ROWS) == 0) {
-        // groups of 4 rows are one sector each, 1 KB apart (the 32 lanes of the block sit in between)
-        double *q = dst + working_index(t0, k, ldd, tile_rows, n_blocks, 3);
+            for (int r = 0; r < ROWS; r += 4) st256(q + r, v[r], v[r + 1], v[r + 2], v[r + 3]);
+            continue;
+        }
+        if (layout == 3 && (tile_rows % ROWS) == 0) {
+            // groups of 4 rows are one sector each, 1 KB apart (the 32 lanes of the block sit in between)
+            double *q = dst + working_index(t0, k, ldd, tile_rows, n_blocks, 3);
 #pragma unroll
-        for (int r = 0; r < ROWS; r += 4) st256(q + (size_t)(r >> 2) * (RR_BLOCK * 4), v[r], v[r + 1], v[r + 2], v[r + 3]);
-        return;
-    }
+            for (int r = 0; r < ROWS; r += 4) st256(q + (size_t)(r >> 2) * (RR_BLOCK * 4), v[r], v[r + 1], v[r + 2], v[r + 3]);
+            continue;
+        }
 #pragma unroll
-    for (int r = 0; r < ROWS; ++r)
-        if (t0 + r < T) dst[working_index(t0 + r, k, ldd, tile_rows, n_blocks, layout)] = v[r];
+        for (int r = 0; r < ROWS; ++r)
+            if (t0 + r < T) dst[working_index(t0 + r, k, ldd, tile_rows, n_blocks, layout)] = v[r];
+    } while (STRIDE && (t0 += (int64_t)gridDim.y * ROWS) < T);
 }
-template <int ROWS>
+template <int ROWS, bool STRIDE>
 __global__ void __launch_bounds__(256) permute_to_user(const double *__restrict__ src, int64_t lds, double *__restrict__ dst,
                                                        int64_t ldd, const int32_t *__restrict__ inv, int64_t n, int64_t T,
                                                        int64_t tile_rows, int64_t n_blocks, int layout, int clamp) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int64_t k = __ldg(inv + i);
-    const int64_t t0 = (int64_t)blockIdx.y * ROWS;
-    double v[ROWS];
-    if (layout == 2 && (tile_rows % ROWS) == 0) {
-        const double *q = src + working_index(t0, k, lds, tile_rows, n_blocks, 2);
+    int64_t t0 = (int64_t)blockIdx.y * ROWS;
+    do {
+        double v[ROWS];
+        if (layout == 2 && (tile_rows % ROWS) == 0) {
+            const double *q = src + working_index(t0, k, lds, tile_rows, n_blocks, 2);
 #pragma unroll
-        for (int r = 0; r < ROWS; r += 4) ld256(q + r, v[r], v[r + 1], v[r + 2], v[r + 3]);
-    } else {
+            for (int r = 0; r < ROWS; r += 4) ld256(q + r, v[r], v[r + 1], v[r + 2], v[r + 3]);
+        } else {
+#pragma unroll
+            for (int r = 0; r < ROWS; ++r)
+                v[r] = (t0 + r < T) ? src[working_index(t0 + r, k, lds, tile_rows, n_blocks, layout)] : 0.0;
+        }
+        if (clamp) {   // direct exchange: the working array holds the raw series; the reference's clamp (_numba_kernels.py:44-46, :82-84)
+#pragma unroll
+            for (int r = 0; r < ROWS; ++r) v[r] = v[r] > 0.0 ? v[r] : 0.0;
+        }
 #pragma unroll
         for (int r = 0; r < ROWS; ++r)
-            v[r] = (t0 + r < T) ? src[working_index(t0 + r, k, lds, tile_rows, n_blocks, layout)] : 0.0;
-    }
-    if (clamp) {   // direct exchange: the working array holds the raw series; the reference's clamp (_numba_kernels.py:44-46, :82-84)
-#pragma unroll
-        for (int r = 0; r < ROWS; ++r) v[r] = v[r] > 0.0 ? v[r] : 0.0;
-    }
-#pragma unroll
-    for (int r = 0; r < ROWS; ++r)
-        if (t0 + r < T) dst[(t0 + r) * ldd + i] = v[r];
+            if (t0 + r < T) dst[(t0 + r) * ldd + i] = v[r];
+    } while (STRIDE && (t0 += (int64_t)gridDim.y * ROWS) < T);
 }
 static int permute(bool to_working, const double *src, int64_t lds, double *dst, int64_t ldd, const int32_t *inv,
                    int64_t n, int64_t T, cudaStream_t stream, int64_t tile_rows = 0, int64_t n_blocks = 0, int layout = 0,
                    int clamp = 0) {
     rr_timer tm(to_working ? 1 : 2, stream);
     const unsigned gx = (unsigned)((n + 255) / 256);
-    if (to_working && (layout == 2 || layout == 3) && (tile_rows % 16) == 0) {
-        dim3 grid(gx, (unsigned)((T + 15) / 16));
-        permute_to_working<16><<<grid, 256, 0, stream>>>(src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout);
-    } else if (to_working) {
-        dim3 grid(gx, (unsigned)((T + PERM_ROWS - 1) / PERM_ROWS));
-        permute_to_working<PERM_ROWS><<<grid, 256, 0, stream>>>(src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout);
-    } else if (layout == 2 && (tile_rows % 16) == 0) {
-        dim3 grid(gx, (unsigned)((T + 15) / 16));
-        permute_to_user<16><<<grid, 256, 0, stream>>>(src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout, clamp);
-    } else {
-        dim3 grid(gx, (unsigned)((T + PERM_ROWS - 1) / PERM_ROWS));
-        permute_to_user<PERM_ROWS><<<grid, 256, 0, stream>>>(src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout, clamp);
-    }
+    // one grid row per group of rows, at most 65535: past that the CTAs stride over the rest (the striding instantiations
+    // are separate so that shorter calls keep the registers, and the occupancy, of one row group per CTA)
+    auto rows_grid = [&](int64_t rows) { return dim3(gx, (unsigned)std::min<int64_t>((T + rows - 1) / rows, 65535)); };
+#define PERMUTE(KERNEL, ROWS, ...) do {                                                                               \
+        if ((T + ROWS - 1) / ROWS > 65535) KERNEL<ROWS, true><<<rows_grid(ROWS), 256, 0, stream>>>(__VA_ARGS__);       \
+        else KERNEL<ROWS, false><<<rows_grid(ROWS), 256, 0, stream>>>(__VA_ARGS__);                                    \
+    } while (0)
+    if (to_working && (layout == 2 || layout == 3) && (tile_rows % 16) == 0)
+        PERMUTE(permute_to_working, 16, src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout);
+    else if (to_working)
+        PERMUTE(permute_to_working, PERM_ROWS, src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout);
+    else if (layout == 2 && (tile_rows % 16) == 0)
+        PERMUTE(permute_to_user, 16, src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout, clamp);
+    else
+        PERMUTE(permute_to_user, PERM_ROWS, src, lds, dst, ldd, inv, n, T, tile_rows, n_blocks, layout, clamp);
+#undef PERMUTE
     CK(cudaGetLastError());
     rr_count_launch(1);
     return 0;

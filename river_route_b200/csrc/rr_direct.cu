@@ -903,9 +903,13 @@ __global__ void __launch_bounds__(256) stage_in_kernel(const ST *__restrict__ sr
     if (hw) q_final[k] = q;
 }
 
+// The stage_out kernels take one row group (or time tile) per grid row.  grid.y is capped at 65535; a call with more
+// groups launches the STRIDE instantiation, whose CTAs stride over them by gridDim.y.  Without STRIDE the loop body runs
+// once and compiles to the one-group-per-CTA code, with its registers and occupancy.
+
 // working discharge tiles -> caller's rows: column s of the output shows segment subset[s] (or s); clamp as the
 // reference does on the interval mean (K == 1: the value itself); OT = float rounds like numpy's astype(float32)
-template <typename OT>
+template <typename OT, bool STRIDE>
 __global__ void __launch_bounds__(256) stage_out_kernel(const double *__restrict__ out_w, OT *__restrict__ dst, int64_t ldd,
                                                         const int32_t *__restrict__ inv, const int32_t *__restrict__ subset,
                                                         int64_t n_out, int64_t T, int64_t tile_rows, int64_t pitch,
@@ -914,25 +918,27 @@ __global__ void __launch_bounds__(256) stage_out_kernel(const double *__restrict
     if (s >= n_out) return;
     const int64_t i = subset ? (int64_t)__ldg(subset + s) : s;
     const int64_t k = __ldg(inv + i);
-    const int64_t t0 = (int64_t)blockIdx.y * 16;
-    const double *p = out_w + tile_index(t0, k, tile_rows, pitch, n_blocks);
-    double v[16];
+    int64_t t0 = (int64_t)blockIdx.y * 16;
+    do {
+        const double *p = out_w + tile_index(t0, k, tile_rows, pitch, n_blocks);
+        double v[16];
 #pragma unroll
-    for (int r = 0; r < 16; r += 4) {
-        const d4 x = ld_sector_ro(p + r);
-        v[r] = x.a; v[r + 1] = x.b; v[r + 2] = x.c; v[r + 3] = x.d;
-    }
-#pragma unroll
-    for (int r = 0; r < 16; ++r)
-        if (t0 + r < T) {
-            const double val = v[r] > 0.0 ? v[r] : 0.0;              // _numba_kernels.py:44-46 / :82-84
-            dst[(t0 + r) * ldd + s] = (OT)val;
+        for (int r = 0; r < 16; r += 4) {
+            const d4 x = ld_sector_ro(p + r);
+            v[r] = x.a; v[r + 1] = x.b; v[r + 2] = x.c; v[r + 3] = x.d;
         }
+#pragma unroll
+        for (int r = 0; r < 16; ++r)
+            if (t0 + r < T) {
+                const double val = v[r] > 0.0 ? v[r] : 0.0;              // _numba_kernels.py:44-46 / :82-84
+                dst[(t0 + r) * ldd + s] = (OT)val;
+            }
+    } while (STRIDE && (t0 += (int64_t)gridDim.y * 16) < T);
 }
 
 // More than one routing substep per row: the tiles hold the raw substep series; an output row is the clamped mean of its K
 // substeps, accumulated in substep order and multiplied by 1/K exactly as _numba_kernels.py:19, :41-46 / :60, :79-84 do.
-template <typename OT>
+template <typename OT, bool STRIDE>
 __global__ void __launch_bounds__(256) stage_out_sub_kernel(const double *__restrict__ out_w, OT *__restrict__ dst, int64_t ldd,
                                                             const int32_t *__restrict__ inv, const int32_t *__restrict__ subset,
                                                             int64_t n_out, int64_t T, int64_t tile_rows, int64_t pitch,
@@ -941,22 +947,25 @@ __global__ void __launch_bounds__(256) stage_out_sub_kernel(const double *__rest
     if (s >= n_out) return;
     const int64_t i = subset ? (int64_t)__ldg(subset + s) : s;
     const int64_t k = __ldg(inv + i);
-    const int64_t j = blockIdx.y;                                            // one time tile per grid row
-    const double *p = out_w + ((j * n_blocks + (k >> 5)) * RR_BLOCK + (k & 31)) * pitch;
     const double inv_k = 1.0 / (double)K;
-    const int64_t t0 = j * tile_rows, rows = min(tile_rows, T - t0);
-    for (int64_t r = 0; r < rows; ++r) {
-        double acc = 0.0;
-        for (int q = 0; q < K; ++q) acc += p[r * K + q];
-        const double val = acc * inv_k;
-        dst[(t0 + r) * ldd + s] = (OT)(val > 0.0 ? val : 0.0);
-    }
+    const int64_t n_tiles = (T + tile_rows - 1) / tile_rows;
+    int64_t j = blockIdx.y;
+    do {   // one time tile per grid row
+        const double *p = out_w + ((j * n_blocks + (k >> 5)) * RR_BLOCK + (k & 31)) * pitch;
+        const int64_t t0 = j * tile_rows, rows = min(tile_rows, T - t0);
+        for (int64_t r = 0; r < rows; ++r) {
+            double acc = 0.0;
+            for (int q = 0; q < K; ++q) acc += p[r * K + q];
+            const double val = acc * inv_k;
+            dst[(t0 + r) * ldd + s] = (OT)(val > 0.0 ? val : 0.0);
+        }
+    } while (STRIDE && (j += gridDim.y) < n_tiles);
 }
 
 // UnitMuskingum: the discharge tiles hold q_ch of the inner reaches.  Output = the convolved lateral inflow itself for
 // headwaters (unclamped, _numba_kernels.py:122-123), max(q_ch + lateral, 0) for inner reaches (:165-171, one substep
 // per row); the lateral rows are read from the caller's array (coalesced, column i = segment i).
-template <typename OT>
+template <typename OT, bool STRIDE>
 __global__ void __launch_bounds__(256) stage_out_unit_kernel(const double *__restrict__ out_w, const double *__restrict__ lat,
                                                              int64_t ldl, OT *__restrict__ dst, int64_t ldd,
                                                              const int32_t *__restrict__ inv, const int32_t *__restrict__ subset,
@@ -966,27 +975,29 @@ __global__ void __launch_bounds__(256) stage_out_unit_kernel(const double *__res
     if (s >= n_out) return;
     const int64_t i = subset ? (int64_t)__ldg(subset + s) : s;
     const int64_t k = __ldg(inv + i);
-    const int64_t t0 = (int64_t)blockIdx.y * 16;
     const bool hw = k < hw_slots;
-    double v[16];
+    int64_t t0 = (int64_t)blockIdx.y * 16;
+    do {
+        double v[16];
 #pragma unroll
-    for (int r = 0; r < 16; ++r) v[r] = 0.0;
-    if (!hw) {
-        const double *p = out_w + tile_index(t0, k, tile_rows, pitch, n_blocks);
+        for (int r = 0; r < 16; ++r) v[r] = 0.0;
+        if (!hw) {
+            const double *p = out_w + tile_index(t0, k, tile_rows, pitch, n_blocks);
 #pragma unroll
-        for (int r = 0; r < 16; r += 4) {
-            const d4 x = ld_sector_ro(p + r);
-            v[r] = x.a; v[r + 1] = x.b; v[r + 2] = x.c; v[r + 3] = x.d;
+            for (int r = 0; r < 16; r += 4) {
+                const d4 x = ld_sector_ro(p + r);
+                v[r] = x.a; v[r + 1] = x.b; v[r + 2] = x.c; v[r + 3] = x.d;
+            }
         }
-    }
 #pragma unroll
-    for (int r = 0; r < 16; ++r)
-        if (t0 + r < T) {
-            const double l = __ldg(lat + (t0 + r) * ldl + i);
-            double val = l;
-            if (!hw) { val = v[r] + l; val = val > 0.0 ? val : 0.0; }
-            dst[(t0 + r) * ldd + s] = (OT)val;
-        }
+        for (int r = 0; r < 16; ++r)
+            if (t0 + r < T) {
+                const double l = __ldg(lat + (t0 + r) * ldl + i);
+                double val = l;
+                if (!hw) { val = v[r] + l; val = val > 0.0 ? val : 0.0; }
+                dst[(t0 + r) * ldd + s] = (OT)val;
+            }
+    } while (STRIDE && (t0 += (int64_t)gridDim.y * 16) < T);
 }
 
 // UnitMuskingum state hand-back in the caller's order.  last != 0: the recombined vector of UnitMuskingum.py:94-98
@@ -1019,21 +1030,27 @@ __global__ void __launch_bounds__(256) unit_state_kernel(const double *__restric
     } while (0)
 
 // Discharge tiles of the narrow blocks of one member <- the "not written yet" pattern (narrow_item).  One CTA per
-// (narrow block, tile): the block's tile is 32 x pitch contiguous doubles.
+// (narrow block, tile): the block's tile is 32 x pitch contiguous doubles.  grid.y is capped at 65535: with more tiles
+// a CTA strides over them (STRIDE).
+template <bool STRIDE>
 __global__ void __launch_bounds__(256) fill_sentinel_kernel(double *__restrict__ out_w, const int32_t *__restrict__ narrow_blocks,
-                                                            int32_t first_block, int64_t n_blocks, int64_t pitch) {
+                                                            int32_t first_block, int64_t n_blocks, int64_t n_tiles, int64_t pitch) {
     const int32_t b = __ldg(narrow_blocks + blockIdx.x);
     if (b < first_block) return;
-    double *p = out_w + (((size_t)blockIdx.y * n_blocks + (size_t)b) * RR_BLOCK) * (size_t)pitch;
     const double sv = __longlong_as_double((long long)RR_SENTINEL_BITS);
-    for (int64_t e = (int64_t)threadIdx.x * 4; e < RR_BLOCK * pitch; e += 256 * 4) st_sector(p + e, sv, sv, sv, sv);
+    int64_t j = blockIdx.y;
+    do {
+        double *p = out_w + (((size_t)j * n_blocks + (size_t)b) * RR_BLOCK) * (size_t)pitch;
+        for (int64_t e = (int64_t)threadIdx.x * 4; e < RR_BLOCK * pitch; e += 256 * 4) st_sector(p + e, sv, sv, sv, sv);
+    } while (STRIDE && (j += gridDim.y) < n_tiles);
 }
 
 int rr_fill_sentinel(double *out_w, const int32_t *narrow_blocks, int64_t n_narrow, int64_t first_block, int64_t n_blocks,
                      int64_t n_tiles, int64_t pitch, cudaStream_t stream) {
     if (n_narrow <= 0) return 0;
-    dim3 grid((unsigned)n_narrow, (unsigned)n_tiles);
-    fill_sentinel_kernel<<<grid, 256, 0, stream>>>(out_w, narrow_blocks, (int32_t)first_block, n_blocks, pitch);
+    dim3 grid((unsigned)n_narrow, (unsigned)std::min<int64_t>(n_tiles, 65535));
+    if (n_tiles > 65535) fill_sentinel_kernel<true><<<grid, 256, 0, stream>>>(out_w, narrow_blocks, (int32_t)first_block, n_blocks, n_tiles, pitch);
+    else fill_sentinel_kernel<false><<<grid, 256, 0, stream>>>(out_w, narrow_blocks, (int32_t)first_block, n_blocks, n_tiles, pitch);
     CKD(cudaGetLastError());
     rr_count_launch(1);
     return 0;
@@ -1064,11 +1081,11 @@ int rr_stage_in(const void *src, int src_f32, int64_t lds, double *lat_w, double
 int rr_stage_out(const double *out_w, void *dst, int dst_f32, int64_t ldd, const int32_t *inv, const int32_t *subset,
                  int64_t n_out, int64_t T, int64_t tile_rows, int64_t n_blocks, cudaStream_t stream) {
     const int64_t pitch = (tile_rows + 3) & ~(int64_t)3;
-    dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)((T + 15) / 16));
-    if (dst_f32)
-        stage_out_kernel<float><<<grid, 256, 0, stream>>>(out_w, (float *)dst, ldd, inv, subset, n_out, T, tile_rows, pitch, n_blocks);
-    else
-        stage_out_kernel<double><<<grid, 256, 0, stream>>>(out_w, (double *)dst, ldd, inv, subset, n_out, T, tile_rows, pitch, n_blocks);
+    dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)std::min<int64_t>((T + 15) / 16, 65535));
+#define STAGE_OUT(OT, S) stage_out_kernel<OT, S><<<grid, 256, 0, stream>>>(out_w, (OT *)dst, ldd, inv, subset, n_out, T, tile_rows, pitch, n_blocks)
+    if ((T + 15) / 16 > 65535) { if (dst_f32) STAGE_OUT(float, true); else STAGE_OUT(double, true); }
+    else { if (dst_f32) STAGE_OUT(float, false); else STAGE_OUT(double, false); }
+#undef STAGE_OUT
     CKD(cudaGetLastError());
     rr_count_launch(1);
     return 0;
@@ -1078,13 +1095,12 @@ int rr_stage_out_unit(const double *out_w, const double *lat, int64_t ldl, void 
                       const int32_t *subset, int64_t n_out, int64_t T, int64_t tile_rows, int64_t n_blocks, int64_t hw_slots,
                       cudaStream_t stream) {
     const int64_t pitch = (tile_rows + 3) & ~(int64_t)3;
-    dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)((T + 15) / 16));
-    if (dst_f32)
-        stage_out_unit_kernel<float><<<grid, 256, 0, stream>>>(out_w, lat, ldl, (float *)dst, ldd, inv, subset, n_out, T, tile_rows,
-                                                               pitch, n_blocks, hw_slots);
-    else
-        stage_out_unit_kernel<double><<<grid, 256, 0, stream>>>(out_w, lat, ldl, (double *)dst, ldd, inv, subset, n_out, T, tile_rows,
-                                                                pitch, n_blocks, hw_slots);
+    dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)std::min<int64_t>((T + 15) / 16, 65535));
+#define STAGE_OUT(OT, S) stage_out_unit_kernel<OT, S><<<grid, 256, 0, stream>>>(out_w, lat, ldl, (OT *)dst, ldd, inv, subset, n_out, T, \
+                                                                             tile_rows, pitch, n_blocks, hw_slots)
+    if ((T + 15) / 16 > 65535) { if (dst_f32) STAGE_OUT(float, true); else STAGE_OUT(double, true); }
+    else { if (dst_f32) STAGE_OUT(float, false); else STAGE_OUT(double, false); }
+#undef STAGE_OUT
     CKD(cudaGetLastError());
     rr_count_launch(1);
     return 0;
@@ -1100,11 +1116,11 @@ int rr_unit_state_to_user(const double *qs_w, const double *qf_w, const int32_t 
 
 int rr_stage_out_sub(const double *out_w, void *dst, int dst_f32, int64_t ldd, const int32_t *inv, const int32_t *subset,
                      int64_t n_out, int64_t T, int64_t tile_rows, int64_t pitch, int64_t n_blocks, int K, cudaStream_t stream) {
-    dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)((T + tile_rows - 1) / tile_rows));
-    if (dst_f32)
-        stage_out_sub_kernel<float><<<grid, 256, 0, stream>>>(out_w, (float *)dst, ldd, inv, subset, n_out, T, tile_rows, pitch, n_blocks, K);
-    else
-        stage_out_sub_kernel<double><<<grid, 256, 0, stream>>>(out_w, (double *)dst, ldd, inv, subset, n_out, T, tile_rows, pitch, n_blocks, K);
+    dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)std::min<int64_t>((T + tile_rows - 1) / tile_rows, 65535));
+#define STAGE_OUT(OT, S) stage_out_sub_kernel<OT, S><<<grid, 256, 0, stream>>>(out_w, (OT *)dst, ldd, inv, subset, n_out, T, tile_rows, pitch, n_blocks, K)
+    if ((T + tile_rows - 1) / tile_rows > 65535) { if (dst_f32) STAGE_OUT(float, true); else STAGE_OUT(double, true); }
+    else { if (dst_f32) STAGE_OUT(float, false); else STAGE_OUT(double, false); }
+#undef STAGE_OUT
     CKD(cudaGetLastError());
     rr_count_launch(1);
     return 0;

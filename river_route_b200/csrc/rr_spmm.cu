@@ -6,12 +6,11 @@
 // incremental, optional clip at zero, NaN -> 0 and optional multiplication by catchment area.
 // Memory-bound CSR SpMM with time as the dense dimension: one thread per river so the (T, n)
 // output rows are written as coalesced 256-byte segments; the runoff is first re-laid as
-// [time block][cell][8 steps] so that each weight entry reads one full 32-byte sector and one launch per
-// time block gathers from an L2-resident slab.
+// [time block][cell][8 steps] so that each weight entry reads one full 32-byte sector and the CTAs of one
+// time block gather from an L2-resident slab.
 #include <cuda_runtime.h>
 
 #include <algorithm>
-#include <cstdlib>
 #include <string>
 
 #include "rr_internal.h"
@@ -40,23 +39,26 @@ constexpr int TB = 8;   // time steps per register block == one 32-byte sector o
 // 128 / 256 contiguous bytes per row), one whole 32-byte sector (float32; two for float64) written per thread, 1 KB
 // contiguous per warp.  (Round 1 went through a 32 x 33 shared-memory tile: 3.0 TB/s under ncu; no tile is needed when the
 // block of TB steps is what a thread owns.)
-template <typename XT>
+template <typename XT, bool STRIDE>
 __global__ void __launch_bounds__(256) transpose_kernel(const XT *__restrict__ x, int64_t ldx, XT *__restrict__ xt,
                                                         int64_t Tp, int64_t T, int64_t n_points) {
     const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int64_t t0 = (int64_t)blockIdx.y * TB;
-    if (c >= n_points || t0 >= Tp) return;
-    XT v[TB];
+    if (c >= n_points) return;
+    // grid.y is capped at 65535: with more time blocks a CTA strides over them (STRIDE), else it handles one
+    int64_t t0 = (int64_t)blockIdx.y * TB;
+    do {
+        XT v[TB];
 #pragma unroll
-    for (int u = 0; u < TB; ++u) v[u] = (t0 + u < T) ? __ldg(x + (t0 + u) * ldx + c) : XT(0);
-    XT *dst = xt + ((t0 / TB) * n_points + c) * TB;
-    if (sizeof(XT) == 4) {
-        asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst), "f"((float)v[0]), "f"((float)v[1]), "f"((float)v[2]),
-                     "f"((float)v[3]), "f"((float)v[4]), "f"((float)v[5]), "f"((float)v[6]), "f"((float)v[7]) : "memory");
-    } else {
-        asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(dst), "d"((double)v[0]), "d"((double)v[1]), "d"((double)v[2]), "d"((double)v[3]) : "memory");
-        asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(dst + 4), "d"((double)v[4]), "d"((double)v[5]), "d"((double)v[6]), "d"((double)v[7]) : "memory");
-    }
+        for (int u = 0; u < TB; ++u) v[u] = (t0 + u < T) ? __ldg(x + (t0 + u) * ldx + c) : XT(0);
+        XT *dst = xt + ((t0 / TB) * n_points + c) * TB;
+        if (sizeof(XT) == 4) {
+            asm volatile("st.global.v8.f32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(dst), "f"((float)v[0]), "f"((float)v[1]), "f"((float)v[2]),
+                         "f"((float)v[3]), "f"((float)v[4]), "f"((float)v[5]), "f"((float)v[6]), "f"((float)v[7]) : "memory");
+        } else {
+            asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(dst), "d"((double)v[0]), "d"((double)v[1]), "d"((double)v[2]), "d"((double)v[3]) : "memory");
+            asm volatile("st.global.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(dst + 4), "d"((double)v[4]), "d"((double)v[5]), "d"((double)v[6]), "d"((double)v[7]) : "memory");
+        }
+    } while (STRIDE && (t0 += (int64_t)gridDim.y * TB) < Tp);
 }
 
 template <typename XT> struct vec8;
@@ -78,33 +80,27 @@ template <> struct vec8<double> {
 
 // One thread per river, TB outputs in registers; row entries are walked in stored (ascending column)
 // order so every output accumulates in scipy's csr_matvecs order; the tail of runoff.py:309-337 is fused.
-// One launch covers the time steps [t_begin, t_end); grid.y splits them further when there are few rivers.
-// `carry` holds the aggregated value of the last step of the previous launch (cumulative input).
-template <typename XT>
-__global__ void __launch_bounds__(128) weights_kernel(int64_t n_rivers, int64_t n_points, int64_t t_begin, int64_t t_end,
-                                                      int64_t chunk,
+// A CTA handles time block blockIdx.y and, with STRIDE (more than 65535 time blocks: grid.y is capped there), every
+// gridDim.y-th block after it.
+template <typename XT, bool STRIDE>
+__global__ void __launch_bounds__(128) weights_kernel(int64_t n_rivers, int64_t n_points, int64_t T,
                                                       const int32_t *__restrict__ indptr,
                                                       const int32_t *__restrict__ indices,
                                                       const double *__restrict__ w, const XT *__restrict__ xt,
                                                       double *__restrict__ y, int64_t ldy,
                                                       int cumulative, int force_positive,
-                                                      const double *__restrict__ area, int64_t t_skip,
-                                                      double *__restrict__ carry) {
+                                                      const double *__restrict__ area, int64_t t_skip) {
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= n_rivers) return;
-    const int64_t tb = t_begin + (int64_t)blockIdx.y * chunk;
-    const int64_t te = min(t_end, tb + chunk);
     const int p0 = __ldg(indptr + r);
     const int p1 = __ldg(indptr + r + 1);
     const double a = area ? __ldg(area + r) : 1.0;
-    double prev = 0.0;   // aggregated value of the step before this block (cumulative input, runoff.py:310-312)
-    if (cumulative && tb > 0) {
-        if (tb == t_begin) prev = carry[r];
-        else
+    int64_t t0 = (int64_t)blockIdx.y * TB;
+    do {
+        double prev = 0.0;   // aggregated value of the step before this block (cumulative input, runoff.py:310-312)
+        if (cumulative && t0 > 0)
             for (int j = p0; j < p1; ++j)
-                prev = fma(__ldg(w + j), (double)__ldg(xt + (((tb - 1) / TB) * n_points + __ldg(indices + j)) * TB + (tb - 1) % TB), prev);
-    }
-    for (int64_t t0 = tb; t0 < te; t0 += TB) {
+                prev = fma(__ldg(w + j), (double)__ldg(xt + (((t0 - 1) / TB) * n_points + __ldg(indices + j)) * TB + (t0 - 1) % TB), prev);
         double acc[TB];
 #pragma unroll
         for (int u = 0; u < TB; ++u) acc[u] = 0.0;
@@ -119,17 +115,16 @@ __global__ void __launch_bounds__(128) weights_kernel(int64_t n_rivers, int64_t 
         }
 #pragma unroll
         for (int u = 0; u < TB; ++u) {
-            if (t0 + u < te && t0 + u >= t_skip) {   // rows before t_skip only seed `prev` (streamed chunks)
+            if (t0 + u < T && t0 + u >= t_skip) {   // rows before t_skip only seed `prev` (streamed chunks)
                 double q = acc[u];
                 if (cumulative) { if (t0 + u > 0) q = acc[u] - prev; prev = acc[u]; }
                 if ((force_positive & 1) && q < 0.0) q = 0.0;        // :313-314
                 if (!(force_positive & 2) && q != q) q = 0.0;        // :331-333 (bit 1: the caller resamples first, :316-329)
                 if (area) q *= a;                         // :335-336
                 y[(t0 + u - t_skip) * ldy + r] = q;
-            } else if (cumulative && t0 + u < te) prev = acc[u];
+            } else if (cumulative && t0 + u < T) prev = acc[u];
         }
-    }
-    if (cumulative && te == t_end) carry[r] = prev;
+    } while (STRIDE && (t0 += (int64_t)gridDim.y * TB) < T);
 }
 
 template <typename XT>
@@ -138,7 +133,6 @@ int run_weights(int64_t n_rivers, int64_t n_points, int64_t T, const int32_t *in
                 const double *area, int64_t t_skip, cudaStream_t stream) {
     const int64_t Tp = ((T + TB - 1) / TB) * TB;
     XT *xt = nullptr;
-    double *carry = nullptr;
     {   // keep the stream-ordered pool's memory between calls (the default trims it at every sync)
         static thread_local int tuned_device = -1;
         int dev = 0;
@@ -153,51 +147,32 @@ int run_weights(int64_t n_rivers, int64_t n_points, int64_t T, const int32_t *in
         }
     }
     CK(cudaMallocAsync((void **)&xt, sizeof(XT) * (size_t)n_points * Tp, stream));
-    if (cumulative) CK(cudaMallocAsync((void **)&carry, sizeof(double) * (size_t)n_rivers, stream));
-    dim3 tg((unsigned)((n_points + 255) / 256), (unsigned)(Tp / TB));
-    transpose_kernel<XT><<<tg, 256, 0, stream>>>(x, ldx, xt, Tp, T, n_points);
+    // one grid row per time block of TB steps, at most 65535: past that the CTAs stride over the rest (the striding
+    // instantiations are separate so that shorter calls keep the registers, and the occupancy, of one block per CTA)
+    const bool stride = Tp / TB > 65535;
+    const unsigned gy = (unsigned)std::min<int64_t>(Tp / TB, 65535);
+    dim3 tg((unsigned)((n_points + 255) / 256), gy);
+    if (stride) transpose_kernel<XT, true><<<tg, 256, 0, stream>>>(x, ldx, xt, Tp, T, n_points);
+    else transpose_kernel<XT, false><<<tg, 256, 0, stream>>>(x, ldx, xt, Tp, T, n_points);
     CK(cudaGetLastError());
     const int threads = 128;
     const unsigned gx = (unsigned)((n_rivers + threads - 1) / threads);
-    int sms = 148, dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     // ONE launch, grid.y = time blocks of TB steps: CTAs are dispatched x-fastest, so the launch sweeps all rivers of one time
     // block before the next and the cells of the block in flight (n_points x 32 B, 33 MB at C3) stay in L2 while they are
     // gathered -- each cell is read by several catchments in no particular order.  (A thread that swept all time steps
     // itself cost 13x the algorithmic DRAM reads; one launch per 32 MB of cells, the round-1 scheme, cost 93 launches of 64 us
-    // with their ramps and tails at C3.)  Cumulative inputs: a block recomputes the aggregate of the step before it.
-    // RR_WEIGHTS_L2_MB selects the launch-per-slab scheme for A/B measurements.
-    int64_t launches = 0;
-    if (getenv("RR_WEIGHTS_L2_MB") == nullptr && (Tp / TB) <= 65535) {
-        dim3 grid(gx, (unsigned)(Tp / TB));
-        weights_kernel<XT><<<grid, threads, 0, stream>>>(n_rivers, n_points, 0, T, TB, indptr, indices, w, xt, y, ldy, cumulative,
-                                                         force_positive, area, t_skip, carry);
-        CK(cudaGetLastError());
-        ++launches;
-    } else {
-    // time steps per launch: the gathered cells of those steps (n_points x steps x element) should stay in L2
-    // (126 MB on B200, shared with the output stream): about 32 MB; everything at once when it is that small
-    int64_t l2_mb = 32;
-    if (const char *env = getenv("RR_WEIGHTS_L2_MB")) l2_mb = std::max(1, atoi(env));
-    int64_t span = std::max<int64_t>(TB, (((l2_mb << 20) / (int64_t)(n_points * sizeof(XT))) / TB) * TB);
-    span = std::min<int64_t>(span, Tp);
-    for (int64_t t_begin = 0; t_begin < T; t_begin += span) {
-        const int64_t t_end = std::min<int64_t>(T, t_begin + span), len = t_end - t_begin;
-        // few rivers: split the span over grid.y so that the machine is filled
-        const int64_t want_y = std::max<int64_t>(1, ((int64_t)sms * 16 + gx - 1) / gx);
-        int64_t chunk = std::max<int64_t>(64, (len + want_y - 1) / want_y);
-        chunk = std::min<int64_t>(((chunk + TB - 1) / TB) * TB, span);
-        dim3 grid(gx, (unsigned)((len + chunk - 1) / chunk));
-        weights_kernel<XT><<<grid, threads, 0, stream>>>(n_rivers, n_points, t_begin, t_end, chunk, indptr, indices, w, xt, y,
-                                                         ldy, cumulative, force_positive, area, t_skip, carry);
-        CK(cudaGetLastError());
-        ++launches;
-    }
-    }
+    // with their ramps and tails at C3.)  Cumulative inputs: a block recomputes the aggregate of the step before it from xt,
+    // which holds every row of the call.
+    dim3 grid(gx, gy);
+    if (stride)
+        weights_kernel<XT, true><<<grid, threads, 0, stream>>>(n_rivers, n_points, T, indptr, indices, w, xt, y, ldy, cumulative,
+                                                               force_positive, area, t_skip);
+    else
+        weights_kernel<XT, false><<<grid, threads, 0, stream>>>(n_rivers, n_points, T, indptr, indices, w, xt, y, ldy, cumulative,
+                                                                force_positive, area, t_skip);
+    CK(cudaGetLastError());
     CK(cudaFreeAsync(xt, stream));
-    if (carry) CK(cudaFreeAsync(carry, stream));
-    rr_count_launch(1 + launches);
+    rr_count_launch(2);
     return 0;
 }
 
